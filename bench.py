@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- LU+IR TFLOP/s (2/3 n^3) of the mixed-precision solver on synthetic diagonally dominant systems.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--n 32768] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--n 32768] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one full solve of one n x n system: no-pivot LU in fp16 (fp32 accumulate) on the tcgen05 tensor cores +
 fp64 iterative refinement to the dsgesv tolerance, inputs (fp64 A, b) already resident in HBM (`value`).  `e2e` is the
@@ -21,6 +21,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only; a benchmark run leaves nothing in it
 PKG_NAME = "mixed-precision_lu_factorization_b200"
 METRIC = "LU+IR TFLOP/s (2/3*n^3)"
 
@@ -78,6 +79,14 @@ class ClockSampler:
         load = sm[len(sm) // 2:] if sm else []
         return dict(sm_mhz=(load[len(load) // 2] if load else None), sm_max_mhz=(max(mx) if mx else None), reasons=reasons,
                     samples=len(sm))
+
+
+def dump_outputs(d, **arrays):
+    """--dump-outputs: what the timed path returned in its last timed step, one DIR/<name>.npy per array."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -276,6 +285,8 @@ def run_distributed(args, m, pk, rank, world, local):
     ms_max, wall_max = float(t[0].item()), float(t[1].item())
     clocks = sampler.stop() if rank == 0 else None
     fwd_err = float((xs[0] - 1).abs().max().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, x=xs[0].cpu().numpy())
 
     extra = dict(per_gpu_tflops=flops(n) / (ms_max * 1e-3) / 1e12 / world)
     if args.extra_n > 0:
@@ -363,7 +374,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--extra-n", type=int, default=65536, help="second workload reported under `extra`: ONE system of this order, which fits a single GPU, solved on the same N GPUs -- the 1 -> 8 curve read on one workload (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps write the solution of the last one as DIR/x.npy (float64, "
+                    "--impl mplu); the inputs come from fixed seeds, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "mplu":
+        ap.error("--dump-outputs needs --impl mplu")
     if args.warmup < 3:
         args.warmup = 3 if args.impl == "mplu" else args.warmup
 
@@ -431,6 +448,8 @@ def main():
     ms_max = float(t.item())
     clocks = sampler.stop() if rank == 0 else None
     fwd_err = float((x - 1).abs().max().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, x=x.cpu().numpy())
 
     # ---- e2e: host buffers through mplu_gesv_host (pinned memory), copies inside the timed region
     e2e = None

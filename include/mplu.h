@@ -173,6 +173,28 @@ int mplu_gesv_device(mplu_context *ctx, int n, const double *dA, long long lda, 
 int mplu_gesv_host(mplu_context *ctx, int n, const double *hA, long long lda, const double *hb, double *hx,
                    const mplu_options *opts, mplu_stats *stats);
 
+/* ---- several right-hand sides: A X = B (LAPACK dsgesv's NRHS / B / LDB / X / LDX) ----
+ * B and X are column-major n x nrhs (leading dimensions ldb, ldx >= n) in the memory space of the variant.  B is not
+ * modified; rows n .. ldx-1 of X are not written.  The regions spanned by B and X must not overlap (MPLU_E_ARG).
+ * Refinement runs over the block like dsgesv: every column is refined until all columns meet the stopping rule of the
+ * single-vector solve (or max_iters).  A column's result does not depend on its position in B or on the other columns;
+ * the columns share only the iteration count.  A and the factors are streamed once per block of columns.
+ * opts.refinement = MPLU_REFINE_GMRES runs the Krylov correction column by column (not batched).
+ * nrhs = 1 is exactly mplu_solve_device / mplu_gesv_device / mplu_gesv_host.
+ * berr: null, or a host array of nrhs doubles receiving each column's backward error ||r_j|| / (||A|| ||x_j|| + ||b_j||)
+ * (infinity norms; 0 for a column solved exactly, e.g. a zero column).
+ * mplu_stats for nrhs > 1: iters is shared by all columns; converged = every column converged; backward_error and
+ * first_backward_error are maxima over the columns; rnorm_inf, xnorm_inf and bnorm_inf are those of the worst column. */
+int mplu_solve_device_nrhs(mplu_context *ctx, int nrhs, const double *dA, long long lda, const double *dB, long long ldb,
+                           double *dX, long long ldx, double *berr, mplu_stats *stats);
+int mplu_gesv_device_nrhs(mplu_context *ctx, int n, int nrhs, const double *dA, long long lda, const double *dB,
+                          long long ldb, double *dX, long long ldx, const mplu_options *opts, double *berr,
+                          mplu_stats *stats);
+/* B is copied to the device alongside A (block column by block column with opts.stream_host), X is copied back */
+int mplu_gesv_host_nrhs(mplu_context *ctx, int n, int nrhs, const double *hA, long long lda, const double *hB,
+                        long long ldb, double *hX, long long ldx, const mplu_options *opts, double *berr,
+                        mplu_stats *stats);
+
 /* Copy the fp32 L\U factors (unit-lower L below the diagonal, U on/above: the dgetrf layout MPF returns) widened
  * to fp64 into a column-major n x n array; `on_device` selects the destination memory space. */
 int mplu_get_factors(mplu_context *ctx, double *LU, long long ldlu, int on_device);

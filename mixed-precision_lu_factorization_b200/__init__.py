@@ -77,13 +77,18 @@ def load_library(path: os.PathLike | None = None) -> C.CDLL:
     lib.mplu_gesv_device.argtypes = [vp, i, vp, ll, vp, vp, C.POINTER(Options), C.POINTER(Stats)]
     lib.mplu_gesv_host.argtypes = [vp, i, vp, ll, vp, vp, C.POINTER(Options), C.POINTER(Stats)]
     lib.mplu_get_factors.argtypes = [vp, vp, ll, i]
+    dp = C.POINTER(C.c_double)
+    lib.mplu_solve_device_nrhs.argtypes = [vp, i, vp, ll, vp, ll, vp, ll, dp, C.POINTER(Stats)]
+    lib.mplu_gesv_device_nrhs.argtypes = [vp, i, i, vp, ll, vp, ll, vp, ll, C.POINTER(Options), dp, C.POINTER(Stats)]
+    lib.mplu_gesv_host_nrhs.argtypes = lib.mplu_gesv_device_nrhs.argtypes
     lib.mplu_gemm16.argtypes = [i, i, i, i, i, f, vp, ll, vp, ll, f, vp, ll, vp, ll, f, i, vp]
     lib.mplu_diag_lu128.argtypes = [vp, ll, vp, vp, vp]
     lib.mplu_residual.argtypes = [i, vp, ll, vp, vp, vp, vp, vp]
     lib.mplu_generate.argtypes = [i, C.c_ulonglong, i, vp, ll, vp, vp]
     lib.mplu_generate.restype = i
     for name in ("mplu_create", "mplu_factor_device", "mplu_solve_device", "mplu_gesv_device", "mplu_gesv_host",
-                 "mplu_get_factors", "mplu_gemm16", "mplu_diag_lu128", "mplu_residual"):
+                 "mplu_get_factors", "mplu_gemm16", "mplu_diag_lu128", "mplu_residual", "mplu_solve_device_nrhs",
+                 "mplu_gesv_device_nrhs", "mplu_gesv_host_nrhs"):
         getattr(lib, name).restype = i
     lib.mplu_MPF.argtypes = [vp, i, i, vp]
     lib.mplu_MPF.restype = i
@@ -122,6 +127,11 @@ def default_options(**kw) -> Options:
             raise TypeError(f"unknown option {k}")
         setattr(o, k, v)
     return o
+
+
+def _dptr(a):
+    """numpy float64 array -> double* for ctypes"""
+    return a.ctypes.data_as(C.POINTER(C.c_double))
 
 
 def _check(code: int, where: str, allow=()):
@@ -175,6 +185,31 @@ class Solver:
                "mplu_gesv_host", allow=(-7,) if allow_noconv else ())
         return st
 
+    # several right-hand sides: B / X column-major n x nrhs (leading dimensions ldb / ldx); returns (Stats, berr), berr a
+    # numpy array of the nrhs per-column backward errors
+    def solve_nrhs_ptr(self, nrhs, dA, lda, dB, ldb, dX, ldx, allow_noconv=False):
+        import numpy as np
+        st, berr = Stats(), np.zeros(max(nrhs, 1))
+        _check(self._lib.mplu_solve_device_nrhs(self._ctx, nrhs, dA, lda, dB, ldb, dX, ldx, _dptr(berr), C.byref(st)),
+               "mplu_solve_device_nrhs", allow=(-7,) if allow_noconv else ())
+        return st, berr[:nrhs]
+
+    def gesv_nrhs_ptr(self, n, nrhs, dA, lda, dB, ldb, dX, ldx, opts=None, allow_noconv=False):
+        import numpy as np
+        st, berr = Stats(), np.zeros(max(nrhs, 1))
+        _check(self._lib.mplu_gesv_device_nrhs(self._ctx, n, nrhs, dA, lda, dB, ldb, dX, ldx, C.byref(opts) if opts else None,
+                                                _dptr(berr), C.byref(st)), "mplu_gesv_device_nrhs",
+               allow=(-7,) if allow_noconv else ())
+        return st, berr[:nrhs]
+
+    def gesv_host_nrhs_ptr(self, n, nrhs, hA, lda, hB, ldb, hX, ldx, opts=None, allow_noconv=False):
+        import numpy as np
+        st, berr = Stats(), np.zeros(max(nrhs, 1))
+        _check(self._lib.mplu_gesv_host_nrhs(self._ctx, n, nrhs, hA, lda, hB, ldb, hX, ldx, C.byref(opts) if opts else None,
+                                              _dptr(berr), C.byref(st)), "mplu_gesv_host_nrhs",
+               allow=(-7,) if allow_noconv else ())
+        return st, berr[:nrhs]
+
     # torch conveniences (column-major convention: pass A.t().contiguous() storage, i.e. a tensor whose memory is
     # column-major; helpers below take "colmajor" tensors of shape (n, n) created with torch.empty(n, n).t()) -----
     def gesv(self, A_cm, b, opts=None, allow_noconv=False):
@@ -187,6 +222,19 @@ class Solver:
         torch.cuda.synchronize(A_cm.device)
         st = self.gesv_ptr(n, A_cm.data_ptr(), lda, b.data_ptr(), x.data_ptr(), opts, allow_noconv)
         return x, st
+
+    def gesv_nrhs(self, A_cm, B_cm, opts=None, allow_noconv=False):
+        """A X = B.  A_cm (n x n) and B_cm (n x nrhs): torch fp64 CUDA tensors with column-major storage.  Returns
+        (X, stats, berr): X column-major n x nrhs, berr a numpy array of the per-column backward errors."""
+        import torch
+        n, nrhs = B_cm.shape
+        assert A_cm.dtype == torch.float64 and A_cm.is_cuda and A_cm.stride(0) == 1 and A_cm.shape == (n, n)
+        assert B_cm.dtype == torch.float64 and B_cm.is_cuda and B_cm.stride(0) == 1
+        X = torch.empty(nrhs, n, dtype=torch.float64, device=A_cm.device).t()  # column-major storage
+        torch.cuda.synchronize(A_cm.device)
+        st, berr = self.gesv_nrhs_ptr(n, nrhs, A_cm.data_ptr(), A_cm.stride(1), B_cm.data_ptr(), max(B_cm.stride(1), n),
+                                      X.data_ptr(), n, opts, allow_noconv)
+        return X, st, berr
 
     def factors(self, n):
         import torch

@@ -51,8 +51,8 @@ __global__ void scale_to_kernel(const double* __restrict__ w, double a, double* 
 
 namespace mplu_detail {
 
-// One GMRES solve of A d = r (r = c->r), x += d.  Returns 0 or an error code; *inner = Krylov steps taken.
-int gmres_correction(mplu_context* c, const double* dA, long long lda, double* dx, int* inner) {
+// One GMRES solve of A d = r (r: n doubles on the device), x += d.  Returns 0 or an error code; *inner = Krylov steps taken.
+int gmres_correction(mplu_context* c, const double* dA, long long lda, const double* r, double* dx, int* inner) {
     const int n = c->n, npad = c->npad;
     const long long ld = npad;
     cudaStream_t st = c->stream;
@@ -87,7 +87,7 @@ int gmres_correction(mplu_context* c, const double* dA, long long lda, double* d
     };
 
     // z0 = (LU)^-1 r -> V[:,0]
-    CKI(launch_lu_solve(c->W, ld, n, npad, c->Linv32, c->Uinv32, c->r, c->y, w, nullptr, c->ready, st));
+    CKI(launch_lu_solve(c->W, ld, n, npad, c->Linv32, c->Uinv32, r, c->y, w, nullptr, c->ready, st));
     CKI(dots(w, 0, hh.data()));
     const double beta = std::sqrt(hh[0]);
     *inner = 0;

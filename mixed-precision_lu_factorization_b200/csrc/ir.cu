@@ -386,6 +386,296 @@ lu_solve_kernel(const float* __restrict__ W_, long long ldw, int n, int nblk, co
     if (use_mbox) ptx::cluster_sync_all();  // no CTA leaves while a neighbour may still store into its mailbox
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Several right-hand sides.  The single-vector kernels above read all of A (residual) or all of the factors (solve)
+// for ONE column; these read them once for a block of columns.  A column's arithmetic is the same whatever its
+// position in the block, the block's width or the other columns: the same products summed in the same order.
+
+constexpr int RB_THREADS = 128;  // each thread owns 2 consecutive rows, as in residual_partial_kernel
+constexpr int RB_TILE = 128;     // columns of A whose X entries are staged in shared memory at a time
+
+__device__ __forceinline__ double nan_max(double a, double b) { return (a > b || a != a) ? a : b; }
+
+// partial[(chunk * kstride + j) * n + row] = sum_{c in chunk} A(row,c) * X(c,j) for the kc <= K columns of this block:
+// every entry of A is loaded once for all of them.  kAbs: abs_partial[chunk * n + row] = sum |A(row,c)| as well.
+template <bool kAbs, int K>
+__global__ void __launch_bounds__(RB_THREADS)
+residual_block_partial_kernel(const double* __restrict__ A, long long lda, int n, const double* __restrict__ X,
+                              long long ldx, int kc, double* __restrict__ partial, int kstride, int cols_per,
+                              double* __restrict__ abs_partial) {
+    __shared__ __align__(16) double xs[RB_TILE][K];
+    const int c0 = blockIdx.y * cols_per;
+    const int c1 = min(n, c0 + cols_per);
+    const int r0 = 2 * (blockIdx.x * RB_THREADS + threadIdx.x);
+    const bool vec = (r0 + 1 < n) && ((lda & 1) == 0) && ((reinterpret_cast<uintptr_t>(A) & 15) == 0);
+    double a0[K], a1[K];
+#pragma unroll
+    for (int j = 0; j < K; ++j) a0[j] = a1[j] = 0.0;
+    double s0 = 0.0, s1 = 0.0;
+    for (int cb = c0; cb < c1; cb += RB_TILE) {
+        const int nc = min(RB_TILE, c1 - cb);
+        __syncthreads();  // the previous tile's X entries are consumed
+        for (int e = threadIdx.x; e < RB_TILE * K; e += RB_THREADS) {
+            const int c = e % RB_TILE, j = e / RB_TILE;
+            xs[c][j] = (c < nc && j < kc) ? X[cb + c + (long long)j * ldx] : 0.0;
+        }
+        __syncthreads();
+        if (r0 >= n) continue;
+        const double* Ap = A + r0 + (long long)cb * lda;
+        if (vec) {
+            int c = 0;
+            for (; c + 8 <= nc; c += 8) {
+                double2 v[8];
+#pragma unroll
+                for (int u = 0; u < 8; ++u) v[u] = __ldg(reinterpret_cast<const double2*>(Ap + (long long)(c + u) * lda));
+#pragma unroll
+                for (int u = 0; u < 8; ++u) {
+#pragma unroll
+                    for (int j = 0; j < K; ++j) {
+                        const double xv = xs[c + u][j];
+                        a0[j] = fma(v[u].x, xv, a0[j]);
+                        a1[j] = fma(v[u].y, xv, a1[j]);
+                    }
+                    if (kAbs) { s0 += fabs(v[u].x); s1 += fabs(v[u].y); }
+                }
+            }
+            for (; c < nc; ++c) {
+                const double2 v = __ldg(reinterpret_cast<const double2*>(Ap + (long long)c * lda));
+#pragma unroll
+                for (int j = 0; j < K; ++j) {
+                    a0[j] = fma(v.x, xs[c][j], a0[j]);
+                    a1[j] = fma(v.y, xs[c][j], a1[j]);
+                }
+                if (kAbs) { s0 += fabs(v.x); s1 += fabs(v.y); }
+            }
+        } else {
+            for (int c = 0; c < nc; ++c) {
+                const double v0 = __ldg(Ap + (long long)c * lda);
+                const double v1 = (r0 + 1 < n) ? __ldg(Ap + 1 + (long long)c * lda) : 0.0;
+#pragma unroll
+                for (int j = 0; j < K; ++j) {
+                    a0[j] = fma(v0, xs[c][j], a0[j]);
+                    a1[j] = fma(v1, xs[c][j], a1[j]);
+                }
+                if (kAbs) { s0 += fabs(v0); s1 += fabs(v1); }
+            }
+        }
+    }
+    if (r0 >= n) return;
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        if (j >= kc) break;
+        double* p = partial + ((long long)blockIdx.y * kstride + j) * n + r0;
+        p[0] = a0[j];
+        if (r0 + 1 < n) p[1] = a1[j];
+    }
+    if (kAbs) {
+        abs_partial[(long long)blockIdx.y * n + r0] = s0;
+        if (r0 + 1 < n) abs_partial[(long long)blockIdx.y * n + r0 + 1] = s1;
+    }
+}
+
+// column j = blockIdx.y: R(:,j) = B(:,j) - sum_chunks partial; norms[2j] = max|R(:,j)|, norms[2j+1] = max|X(:,j)|
+// (zeroed by the launcher); abs_partial non-null: *anorm = max_row sum_chunks abs_partial (column 0's blocks do it)
+__global__ void residual_block_finish_kernel(const double* __restrict__ partial, int n, int nchunk, int kstride,
+                                             const double* __restrict__ B, long long ldb, const double* __restrict__ X,
+                                             long long ldx, double* __restrict__ R, long long ldr, double* norms,
+                                             const double* __restrict__ abs_partial, double* anorm) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y;
+    const bool with_abs = abs_partial != nullptr && j == 0;
+    double rv = 0.0, xv = 0.0, av = 0.0;
+    if (i < n) {
+        double s = 0.0;
+        for (int c = 0; c < nchunk; ++c) s += partial[((long long)c * kstride + j) * n + i];
+        if (with_abs)
+            for (int c = 0; c < nchunk; ++c) av += abs_partial[(long long)c * n + i];
+        rv = B[i + (long long)j * ldb] - s;
+        R[i + (long long)j * ldr] = rv;
+        rv = fabs(rv);
+        xv = fabs(X[i + (long long)j * ldx]);
+    }
+    for (int o = 16; o > 0; o >>= 1) {  // a NaN must survive the reduction: it ends the refinement
+        rv = nan_max(rv, __shfl_xor_sync(0xffffffffu, rv, o));
+        xv = nan_max(xv, __shfl_xor_sync(0xffffffffu, xv, o));
+        av = fmax(av, __shfl_xor_sync(0xffffffffu, av, o));
+    }
+    if ((threadIdx.x & 31) == 0) {
+        atomic_max_double_nonneg(&norms[2 * j], rv);
+        atomic_max_double_nonneg(&norms[2 * j + 1], xv);
+        if (with_abs) atomic_max_double_nonneg(anorm, av);
+    }
+}
+
+// out[j] = max_i |B(i,j)|   (zeroed by the launcher), grid (chunks, columns)
+__global__ void column_absmax_kernel(const double* __restrict__ B, long long ldb, int n, double* out) {
+    const int j = blockIdx.y;
+    double m = 0.0;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) m = nan_max(m, fabs(B[i + (long long)j * ldb]));
+    for (int o = 16; o > 0; o >>= 1) m = nan_max(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if ((threadIdx.x & 31) == 0) atomic_max_double_nonneg(&out[j], m);
+}
+
+__device__ __forceinline__ void st_relaxed_f4(float4* p, float4 v) {
+    asm volatile("st.relaxed.gpu.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+}
+__device__ __forceinline__ bool has_nan(float4 v) { return (v.x != v.x) | (v.y != v.y) | (v.z != v.z) | (v.w != v.w); }
+
+// Both triangular sweeps of L U D = R for kc <= TSB_K columns in one cooperative launch: lu_solve_kernel's steps (one
+// 128-row block of one sweep, left-looking, steps complete in order, `ready` counts them, consumers poll the NaN-
+// prefilled data and consult the counter every 64 polls), widened to a block of columns.  Every 128 x 128 factor tile
+// of a block row is loaded once (4 rows x 16 columns per thread, double-buffered in registers, the diagonal block's
+// inverse last) and multiplied into all columns.  The 128 x TSB_K solution blocks are too large for registers: the
+// operand block of each tile is polled from L2 by all 256 threads (one float4 each) into shared memory and read from
+// there as a warp-wide broadcast.  No DSMEM mailboxes: per step there is TSB_K times the arithmetic of the
+// single-vector kernel, so the L2 hand-off latency weighs less on the chain.
+// ysol / xsol: npad x TSB_K fp32, row-interleaved (entry (row, j) at row * TSB_K + j): a solved block is 4 KiB contiguous.
+constexpr int TSB_K = kSolveBlock;
+static_assert(DBS * TSB_K == 4 * TSV_THREADS, "one float4 of a solution block per thread");
+
+__global__ void __launch_bounds__(TSV_THREADS)
+lu_solve_block_kernel(const float* __restrict__ W, long long ldw, int n, int nblk, const float* __restrict__ Linv,
+                      const float* __restrict__ Uinv, const double* __restrict__ rhs, long long ldr, int kc, float* ysol,
+                      float* xsol, double* __restrict__ d_out, long long ldd, double* __restrict__ x_accum, long long ldxa,
+                      unsigned* ready) {
+    __shared__ __align__(16) float s_part[8][DBS][TSB_K];  // per-warp partial products of the block row
+    __shared__ __align__(16) float s_op[2][DBS][TSB_K];    // operand block of the current tile (two buffers)
+    __shared__ __align__(16) float s_acc[DBS][TSB_K];      // right-hand side minus the tile products
+    const int tid = threadIdx.x;
+    const int rg = tid & 31, cg = tid >> 5;          // tile layout: rows 4rg.., columns 16cg..
+    const int orow = tid >> 1, oj = 4 * (tid & 1);   // owner layout: row orow, columns oj .. oj+3 of a block
+    unsigned seen = 0;
+    for (int s = blockIdx.x; s < 2 * nblk; s += gridDim.x) {
+        const bool back = s >= nblk;
+        const int t = back ? s - nblk : s;
+        const int i = back ? nblk - 1 - t : t;
+        const float* solv = back ? xsol : ysol;
+        const float* inv = (back ? Uinv : Linv) + (long long)i * DBS * DBS;
+        const int row = i * DBS + orow;
+        float4 a_pre = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (back) {
+            a_pre = ld_relaxed_f4(reinterpret_cast<const float4*>(ysol) + (long long)i * (DBS * TSB_K / 4) + tid);
+        } else if (row < n) {
+            float a[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) a[u] = (oj + u < kc) ? static_cast<float>(rhs[row + (long long)(oj + u) * ldr]) : 0.f;
+            a_pre = make_float4(a[0], a[1], a[2], a[3]);
+        }
+        float acc[4][TSB_K];
+#pragma unroll
+        for (int r = 0; r < 4; ++r)
+#pragma unroll
+            for (int j = 0; j < TSB_K; ++j) acc[r][j] = 0.f;
+        const float* wrow = W + (long long)i * DBS + 4 * rg;
+        auto load_tile = [&](float4 (&v)[16], int tt) {
+            if (tt < t) {
+                const int j = back ? nblk - 1 - tt : tt;
+                const float* wp = wrow + ((long long)j * DBS + 16 * cg) * ldw;
+#pragma unroll
+                for (int q = 0; q < 16; ++q) v[q] = __ldcs(reinterpret_cast<const float4*>(wp + (long long)q * ldw));
+            } else {
+                const float* ip = inv + 4 * rg + 16 * cg * DBS;
+#pragma unroll
+                for (int q = 0; q < 16; ++q) v[q] = __ldcs(reinterpret_cast<const float4*>(ip + q * DBS));
+            }
+        };
+        // o[r][j] += sum_q v[q].r * blk[16 cg + q][j]
+        auto multiply = [&](const float4 (&v)[16], const float (*blk)[TSB_K], float (&o)[4][TSB_K]) {
+#pragma unroll
+            for (int q = 0; q < 16; ++q) {
+                const float4 lo = *reinterpret_cast<const float4*>(&blk[16 * cg + q][0]);
+                const float4 hi = *reinterpret_cast<const float4*>(&blk[16 * cg + q][4]);
+                const float sv[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+                const float w[4] = {v[q].x, v[q].y, v[q].z, v[q].w};
+#pragma unroll
+                for (int r = 0; r < 4; ++r)
+#pragma unroll
+                    for (int j = 0; j < TSB_K; ++j) o[r][j] = fmaf(w[r], sv[j], o[r][j]);
+            }
+        };
+        // wait for the solution block tile tt multiplies, stage it, accumulate
+        auto consume = [&](const float4 (&v)[16], int tt) {
+            const int j = back ? nblk - 1 - tt : tt;
+            const unsigned need = (back ? nblk : 0) + tt + 1;
+            const float4* sp = reinterpret_cast<const float4*>(solv) + (long long)j * (DBS * TSB_K / 4) + tid;
+            float4 x4;
+            for (int spin = 0;; ++spin) {
+                x4 = ld_relaxed_f4(sp);
+                if (!has_nan(x4) || seen >= need) break;
+                if ((spin & 63) == 63) seen = ld_acquire_u32(ready);  // a NaN that is data, not "not yet written"
+            }
+            reinterpret_cast<float4*>(&s_op[tt & 1][0][0])[tid] = x4;
+            __syncthreads();  // (the buffer written here was last read two tiles ago, before the previous barrier)
+            multiply(v, s_op[tt & 1], acc);
+        };
+        // partial products of the 8 warps -> s_part; the owner of (row, oj..oj+3) adds (sign 1) or subtracts (sign -1)
+        // them in warp order, the order of lu_solve_kernel
+        auto reduce = [&](const float (&o)[4][TSB_K], float4 sum, float sign) {
+#pragma unroll
+            for (int r = 0; r < 4; ++r) {
+                float4* p = reinterpret_cast<float4*>(&s_part[cg][4 * rg + r][0]);
+                p[0] = make_float4(o[r][0], o[r][1], o[r][2], o[r][3]);
+                p[1] = make_float4(o[r][4], o[r][5], o[r][6], o[r][7]);
+            }
+            __syncthreads();
+#pragma unroll
+            for (int g = 0; g < 8; ++g) {
+                const float4 pg = reinterpret_cast<const float4*>(&s_part[g][0][0])[tid];
+                sum.x += sign * pg.x; sum.y += sign * pg.y; sum.z += sign * pg.z; sum.w += sign * pg.w;
+            }
+            return sum;
+        };
+        auto finish = [&](const float4 (&vi)[16]) {
+            float4 a = a_pre;
+            if (back) {  // y of this block row, solved at forward step i of this launch (the prefetch may predate it)
+                for (int spin = 0; has_nan(a); ++spin) {
+                    a = ld_relaxed_f4(reinterpret_cast<const float4*>(ysol) + (long long)i * (DBS * TSB_K / 4) + tid);
+                    if (!has_nan(a) || seen >= (unsigned)(i + 1)) break;  // read after the counter said so: final
+                    if ((spin & 63) == 63) seen = ld_acquire_u32(ready);
+                }
+            }
+            a = reduce(acc, a, -1.f);
+            reinterpret_cast<float4*>(&s_acc[0][0])[tid] = a;
+            __syncthreads();  // s_acc complete; every owner has read s_part
+            float o[4][TSB_K];
+#pragma unroll
+            for (int r = 0; r < 4; ++r)
+#pragma unroll
+                for (int j = 0; j < TSB_K; ++j) o[r][j] = 0.f;
+            multiply(vi, s_acc, o);
+            const float4 v = reduce(o, make_float4(0.f, 0.f, 0.f, 0.f), 1.f);
+            float* sol = back ? xsol : ysol;
+            st_relaxed_f4(reinterpret_cast<float4*>(sol) + (long long)i * (DBS * TSB_K / 4) + tid, v);
+            if (back && row < n) {
+                const float vv[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+                for (int u = 0; u < 4; ++u)
+                    if (oj + u < kc) {
+                        if (d_out) d_out[row + (long long)(oj + u) * ldd] = static_cast<double>(vv[u]);
+                        if (x_accum) x_accum[row + (long long)(oj + u) * ldxa] += static_cast<double>(vv[u]);
+                    }
+            }
+        };
+        {
+            float4 va[16], vb[16];
+            load_tile(va, 0);
+            for (int tt = 0; tt < t; tt += 2) {
+                load_tile(vb, tt + 1);
+                consume(va, tt);
+                if (tt + 1 < t) {
+                    load_tile(va, tt + 2);
+                    consume(vb, tt + 1);
+                }
+            }
+            if (t & 1) finish(vb); else finish(va);
+        }
+        __syncthreads();  // s_part / s_acc / s_op are free for the next step
+        if (tid == 0) {
+            __threadfence();
+            st_release_u32(ready, (unsigned)(s + 1));
+        }
+    }
+}
+
 }  // namespace
 
 int launch_residual(const double* A, long long lda, int n, const double* x, const double* b, double* r,
@@ -508,6 +798,93 @@ int launch_lu_sweep(const float* W, long long ldw, int n, int npad, const float*
                                 s_begin, s_end, use_mbox, sub, pxv, TileChain{});
     }
     return (int)le;
+}
+
+namespace {
+template <bool kAbs, int K>
+void residual_block_partial(dim3 grid, cudaStream_t st, const double* A, long long lda, int n, const double* X, long long ldx,
+                            int kc, double* partial, int cols_per, double* abs_partial) {
+    residual_block_partial_kernel<kAbs, K><<<grid, RB_THREADS, 0, st>>>(A, lda, n, X, ldx, kc, partial, kc, cols_per,
+                                                                        abs_partial);
+}
+template <bool kAbs>
+void residual_block_partial_k(dim3 grid, cudaStream_t st, const double* A, long long lda, int n, const double* X,
+                              long long ldx, int kc, double* partial, int cols_per, double* abs_partial) {
+    // the narrowest instantiation that holds kc columns (a column's sums do not depend on it)
+    if (kc <= 2) residual_block_partial<kAbs, 2>(grid, st, A, lda, n, X, ldx, kc, partial, cols_per, abs_partial);
+    else if (kc <= 4) residual_block_partial<kAbs, 4>(grid, st, A, lda, n, X, ldx, kc, partial, cols_per, abs_partial);
+    else if (kc <= 8) residual_block_partial<kAbs, 8>(grid, st, A, lda, n, X, ldx, kc, partial, cols_per, abs_partial);
+    else residual_block_partial<kAbs, 16>(grid, st, A, lda, n, X, ldx, kc, partial, cols_per, abs_partial);
+}
+}  // namespace
+
+int launch_residual_block(const double* A, long long lda, int n, const double* X, long long ldx, const double* B,
+                          long long ldb, double* R, long long ldr, int kc, double* partial, double* norms, cudaStream_t st,
+                          double* abs_partial, double* anorm) {
+    if (kc < 1 || kc > kResidualBlock) return (int)cudaErrorInvalidValue;
+    const int nchunk = kResidualChunks;
+    const int cols_per = (n + nchunk - 1) / nchunk;
+    const dim3 grid((n + 2 * RB_THREADS - 1) / (2 * RB_THREADS), nchunk);
+    const bool with_abs = abs_partial != nullptr && anorm != nullptr;
+    if (with_abs) {
+        residual_block_partial_k<true>(grid, st, A, lda, n, X, ldx, kc, partial, cols_per, abs_partial);
+        cudaMemsetAsync(anorm, 0, sizeof(double), st);
+    } else {
+        residual_block_partial_k<false>(grid, st, A, lda, n, X, ldx, kc, partial, cols_per, nullptr);
+    }
+    cudaMemsetAsync(norms, 0, 2 * kc * sizeof(double), st);
+    residual_block_finish_kernel<<<dim3((n + 255) / 256, kc), 256, 0, st>>>(partial, n, nchunk, kc, B, ldb, X, ldx,
+                                                                           R, ldr, norms, with_abs ? abs_partial : nullptr,
+                                                                           with_abs ? anorm : nullptr);
+    return (int)cudaGetLastError();
+}
+
+int launch_column_absmax(const double* B, long long ldb, int n, int ncols, double* out, cudaStream_t st) {
+    cudaMemsetAsync(out, 0, ncols * sizeof(double), st);
+    const int chunks = (n + 255) / 256 < 32 ? (n + 255) / 256 : 32;
+    column_absmax_kernel<<<dim3(chunks, ncols), 256, 0, st>>>(B, ldb, n, out);
+    return (int)cudaGetLastError();
+}
+
+int launch_lu_solve_block(const float* W, long long ldw, int n, int npad, const float* Linv32, const float* Uinv32,
+                          const double* rhs, long long ldr, int kc, float* work, double* d_out, long long ldd,
+                          double* x_accum, long long ldxa, unsigned* ready, cudaStream_t st) {
+    if (kc < 1 || kc > TSB_K) return (int)cudaErrorInvalidValue;
+    constexpr int kMaxDev = 64;
+    static int s_max_grid[kMaxDev] = {};
+    static std::mutex s_mu;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= kMaxDev) return (int)cudaErrorInvalidDevice;
+    int max_grid;
+    {
+        std::lock_guard<std::mutex> lock(s_mu);
+        if (!s_max_grid[dev]) {  // every CTA must be resident: consumers spin on steps owned by other CTAs
+            int sms = 0, per_sm = 0;
+            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+            const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lu_solve_block_kernel, TSV_THREADS, 0);
+            if (e != cudaSuccess) return (int)e;
+            if (per_sm < 1) return (int)cudaErrorLaunchOutOfResources;
+            s_max_grid[dev] = sms * per_sm;
+        }
+        max_grid = s_max_grid[dev];
+    }
+    const int nblk = npad / DBS;
+    const long long nw = (long long)npad * TSB_K;
+    float* ysol = work;
+    float* xsol = work + nw;
+    sweep_prep_kernel<<<(unsigned)((nw + 255) / 256), 256, 0, st>>>(ready, 0u, ysol, xsol, (int)nw);
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(nblk < max_grid ? nblk : max_grid);
+    cfg.blockDim = dim3(TSV_THREADS);
+    cfg.stream = st;
+    cudaLaunchAttribute attrs[1];
+    attrs[0].id = cudaLaunchAttributeCooperative;
+    attrs[0].val.cooperative = 1;
+    cfg.attrs = attrs;
+    cfg.numAttrs = 1;
+    return (int)cudaLaunchKernelEx(&cfg, lu_solve_block_kernel, W, ldw, n, nblk, Linv32, Uinv32, rhs, ldr, kc, ysol, xsol,
+                                   d_out, ldd, x_accum, ldxa, ready);
 }
 
 // every tile sweep of a block-cyclic solve in one launch: nb/128 CTAs (one step of each tile sweep per CTA) in clusters of 8,

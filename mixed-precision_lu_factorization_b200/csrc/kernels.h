@@ -54,6 +54,25 @@ int launch_residual(const double* A, long long lda, int n, const double* x, cons
 int launch_lu_solve(const float* W, long long ldw, int n, int npad, const float* Linv32, const float* Uinv32,
                     const double* rhs, float* y, double* d_out, double* x_accum, unsigned* ready, cudaStream_t st);
 
+// Several right-hand sides (column-major blocks).  A column's arithmetic does not depend on its position in the block,
+// on the block's width or on the other columns.
+constexpr int kResidualBlock = 16;  // columns per residual launch (A is streamed once for all of them)
+constexpr int kResidualChunks = 16; // column chunks of A summed separately: workspace kResidualChunks * kc * n
+constexpr int kSolveBlock = 8;      // columns per triangular-solve launch (the factors are streamed once for all of them)
+// R(:, 0..kc) = B - A X in fp64 for kc <= kResidualBlock columns; norms[2j] = ||R(:,j)||_inf, norms[2j+1] = ||X(:,j)||_inf.
+// partial: kResidualChunks * kc * n doubles.  abs_partial (kResidualChunks * n) / anorm non-null: the same pass
+// also forms the row sums of |A| and ||A||_inf
+int launch_residual_block(const double* A, long long lda, int n, const double* X, long long ldx, const double* B,
+                          long long ldb, double* R, long long ldr, int kc, double* partial, double* norms, cudaStream_t st,
+                          double* abs_partial = nullptr, double* anorm = nullptr);
+// out[j] = ||B(:,j)||_inf for ncols columns
+int launch_column_absmax(const double* B, long long ldb, int n, int ncols, double* out, cudaStream_t st);
+// L U D = rhs for kc <= kSolveBlock columns (the arithmetic of launch_lu_solve, column by column); work: 2 * npad *
+// kSolveBlock floats; D (fp64) -> d_out and / or x_accum += D, each column-major with its leading dimension
+int launch_lu_solve_block(const float* W, long long ldw, int n, int npad, const float* Linv32, const float* Uinv32,
+                          const double* rhs, long long ldr, int kc, float* work, double* d_out, long long ldd,
+                          double* x_accum, long long ldxa, unsigned* ready, cudaStream_t st);
+
 // Partial sums that arrive from peer GPUs (block-cyclic solver, csrc/dist.cu): `base` = this rank's exchange buffer (kPxFlagWords
 // flag words, then slots of nb floats); the sweep waits until the Q flags slot0 .. slot0+Q-1 hold `epoch` and subtracts the sum
 // of those slots from its right-hand side.  The launch is already resident (its tile loads under way) when the data lands.

@@ -49,6 +49,26 @@ void free_work(mplu_context* c) {
     c->Linv32 = c->Uinv32 = nullptr; c->cap_nb = 0;
     c->inv_scales = nullptr; c->rowsum_part = nullptr; c->r = c->partial = nullptr; c->y = nullptr;
     c->cap_npad = 0;
+    cudaFree(c->rb_R); cudaFree(c->rb_partial); cudaFree(c->rb_norms); cudaFree(c->rb_y);
+    c->rb_R = c->rb_partial = c->rb_norms = nullptr; c->rb_y = nullptr;
+    c->rb_cap_n = c->rb_cap_npad = c->rb_cap_nrhs = 0;
+}
+
+// workspaces of the multi-column solve, sized for the factored n and nrhs columns (kept and grown across calls)
+int ensure_rhs_work(mplu_context* c, int nrhs) {
+    if (c->rb_R && c->n <= c->rb_cap_n && c->npad <= c->rb_cap_npad && nrhs <= c->rb_cap_nrhs) return 0;
+    const int cap_n = std::max(c->n, c->rb_cap_n), cap_npad = std::max(c->npad, c->rb_cap_npad),
+              cap_nrhs = std::max(nrhs, c->rb_cap_nrhs);
+    cudaFree(c->rb_R); cudaFree(c->rb_partial); cudaFree(c->rb_norms); cudaFree(c->rb_y);
+    c->rb_R = c->rb_partial = c->rb_norms = nullptr; c->rb_y = nullptr;
+    c->rb_cap_n = c->rb_cap_npad = c->rb_cap_nrhs = 0;
+    const size_t kb = (size_t)std::min(cap_nrhs, kResidualBlock);
+    CK(cudaMalloc(&c->rb_R, (size_t)cap_n * cap_nrhs * sizeof(double)));
+    CK(cudaMalloc(&c->rb_partial, (size_t)kResidualChunks * kb * cap_n * sizeof(double)));
+    CK(cudaMalloc(&c->rb_norms, 3 * (size_t)cap_nrhs * sizeof(double)));
+    CK(cudaMalloc(&c->rb_y, 2 * (size_t)cap_npad * kSolveBlock * sizeof(float)));
+    c->rb_cap_n = cap_n; c->rb_cap_npad = cap_npad; c->rb_cap_nrhs = cap_nrhs;
+    return 0;
 }
 
 int effective_nb(const mplu_context* c, int npad) {
@@ -1653,7 +1673,7 @@ int solve_impl(mplu_context* c, const double* dA, long long lda, const double* d
         if (iters >= max_iters) break;
         if (c->opts.refinement == MPLU_REFINE_GMRES) {
             int inner = 0;
-            CKI(gmres_correction(c, dA, lda, dx, &inner));
+            CKI(gmres_correction(c, dA, lda, c->r, dx, &inner));
             gmres_iters += inner;
         } else {
             CKI(launch_lu_solve(c->W, ld, n, npad, c->Linv32, c->Uinv32, c->r, c->y, nullptr, dx, c->ready, st));
@@ -1691,6 +1711,281 @@ int solve_impl(mplu_context* c, const double* dA, long long lda, const double* d
     if (h_status & 1) return MPLU_E_OVERFLOW;
     if (h_status & 2) return MPLU_E_ZEROPIVOT;
     return MPLU_E_NOCONV;
+}
+
+// solve_impl for nrhs > 1 columns: LAPACK dsgesv's refinement over a block.  X0 = (LU)^-1 B, then every column is refined
+// until all of them meet solve_impl's stopping rule (or max_iters): the columns share the iteration count and nothing
+// else.  A and the factors are streamed once per block of kResidualBlock / kSolveBlock columns.  GMRES refinement runs
+// gmres_correction column by column (not batched).
+int solve_nrhs_impl(mplu_context* c, const double* dA, long long lda, int nrhs, const double* dB, long long ldb, double* dX,
+                    long long ldx, double* berr, mplu_stats* stats) {
+    if (!c->factored) return MPLU_E_NOTFACTORED;
+    const int n = c->n, npad = c->npad;
+    const long long ld = npad;
+    cudaStream_t st = c->stream;
+    CKI(ensure_rhs_work(c, nrhs));
+    double* norms = c->rb_norms;               // [2j] ||r_j||_inf, [2j+1] ||x_j||_inf
+    double* bnorms = c->rb_norms + 2 * nrhs;   // [j] ||b_j||_inf
+    CKI(launch_column_absmax(dB, ldb, n, nrhs, bnorms, st));
+    c->kernel_launches += 1;
+    // D = (LU)^-1 rhs for all columns, kSolveBlock at a time: D -> d_out, or x_accum += D
+    auto solve_blocks = [&](const double* rhs, long long ldr, double* d_out, double* x_accum) -> int {
+        for (int j0 = 0; j0 < nrhs; j0 += kSolveBlock) {
+            const int kc = std::min(kSolveBlock, nrhs - j0);
+            CKI(launch_lu_solve_block(c->W, ld, n, npad, c->Linv32, c->Uinv32, rhs + (long long)j0 * ldr, ldr, kc, c->rb_y,
+                                      d_out ? d_out + (long long)j0 * ldx : nullptr, ldx,
+                                      x_accum ? x_accum + (long long)j0 * ldx : nullptr, ldx, c->ready, st));
+            c->kernel_launches += 2;
+        }
+        return 0;
+    };
+    CKI(solve_blocks(dB, ldb, dX, nullptr));
+
+    std::vector<double> h_norms(3 * (size_t)nrhs), be(nrhs), first_be(nrhs);
+    double anorm = 0.0;
+    const double eps = 2.220446049250313e-16 / 2.0;  // LAPACK dlamch('E')
+    int iters = 0, converged = 0, gmres_iters = 0;
+    bool first_pass = true;
+    const int max_iters = c->opts.max_iters > 0 ? c->opts.max_iters : 30;
+    for (;;) {
+        // lazy first touch: ||A||_inf rides in the first residual pass of the first column block
+        const bool with_anorm = c->anorm_pending;
+        for (int j0 = 0; j0 < nrhs; j0 += kResidualBlock) {
+            const int kc = std::min(kResidualBlock, nrhs - j0);
+            const bool abs_here = with_anorm && j0 == 0;
+            CKI(launch_residual_block(dA, lda, n, dX + (long long)j0 * ldx, ldx, dB + (long long)j0 * ldb, ldb,
+                                      c->rb_R + (long long)j0 * n, n, kc, c->rb_partial, norms + 2 * j0, st,
+                                      abs_here ? c->rowsum_part : nullptr, abs_here ? c->anorm : nullptr));
+            c->kernel_launches += 2;
+        }
+        c->anorm_pending = false;
+        CK(cudaMemcpyAsync(h_norms.data(), norms, 3 * (size_t)nrhs * sizeof(double), cudaMemcpyDeviceToHost, st));
+        if (first_pass || with_anorm) CK(cudaMemcpyAsync(&anorm, c->anorm, sizeof(double), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        bool all = true, nan = false;
+        for (int j = 0; j < nrhs; ++j) {
+            const double rn = h_norms[2 * j], xn = h_norms[2 * j + 1], bn = h_norms[2 * nrhs + j];
+            be[j] = backward_error(rn, anorm, xn, bn);
+            if (first_pass) first_be[j] = be[j];
+            const double thresh = c->opts.tol > 0 ? c->opts.tol * anorm * xn : xn * anorm * eps * std::sqrt((double)n);
+            if (!(rn == rn)) nan = true;
+            if (!(rn <= thresh)) all = false;
+        }
+        first_pass = false;
+        if (nan) break;  // NaN: give up
+        if (all) { converged = 1; break; }
+        if (iters >= max_iters) break;
+        if (c->opts.refinement == MPLU_REFINE_GMRES) {
+            for (int j = 0; j < nrhs; ++j) {
+                int inner = 0;
+                CKI(gmres_correction(c, dA, lda, c->rb_R + (long long)j * n, dX + (long long)j * ldx, &inner));
+                gmres_iters += inner;
+            }
+        } else {
+            CKI(solve_blocks(c->rb_R, n, nullptr, dX));
+        }
+        ++iters;
+    }
+    int h_status = 0;
+    CK(cudaMemcpy(&h_status, c->status, sizeof(int), cudaMemcpyDeviceToHost));
+    if (berr) std::copy(be.begin(), be.end(), berr);
+    if (stats) {
+        int w = 0;  // the worst column (a NaN is worse than anything)
+        for (int j = 1; j < nrhs; ++j)
+            if (be[j] > be[w] || (be[j] != be[j] && be[w] == be[w])) w = j;
+        stats->n = n;
+        stats->iters = iters;
+        stats->converged = converged;
+        stats->status_bits = h_status;
+        stats->anorm_inf = anorm;
+        stats->bnorm_inf = h_norms[2 * nrhs + w];
+        stats->xnorm_inf = h_norms[2 * w + 1];
+        stats->rnorm_inf = h_norms[2 * w];
+        stats->backward_error = be[w];
+        stats->first_backward_error = *std::max_element(first_be.begin(), first_be.end());
+        stats->gemm_launches = c->gemm_launches;
+        stats->kernel_launches = c->kernel_launches;
+        stats->trailing_launches = c->trail_count;
+        stats->trailing_flops = c->trail_flops;
+        stats->trailing_bytes = c->trail_bytes;
+        stats->gmres_iters = gmres_iters;
+        float tms = 0.f;
+        for (int i = 0; i < c->trail_count; ++i) {
+            float ms = 0.f;
+            if (cudaEventElapsedTime(&ms, c->trail_ev[2 * i], c->trail_ev[2 * i + 1]) == cudaSuccess) tms += ms;
+        }
+        stats->trailing_ms = tms;
+    }
+    if (converged) return 0;
+    if (h_status & 1) return MPLU_E_OVERFLOW;
+    if (h_status & 2) return MPLU_E_ZEROPIVOT;
+    return MPLU_E_NOCONV;
+}
+
+// The right-hand sides of one call: nrhs column-major columns of B (ldb) and X (ldx); berr: host array of nrhs or null.
+// nrhs = 1 goes through solve_impl, the single-vector path, unchanged.
+struct RhsBlock {
+    int nrhs;
+    const double* B; long long ldb;
+    double* X; long long ldx;
+    double* berr;
+};
+
+int solve_rhs(mplu_context* c, const double* dA, long long lda, const RhsBlock& b, mplu_stats* stats) {
+    if (b.nrhs == 1) return solve_impl(c, dA, lda, b.B, b.X, stats);
+    return solve_nrhs_impl(c, dA, lda, b.nrhs, b.B, b.ldb, b.X, b.ldx, b.berr, stats);
+}
+
+// factor + solve from device-resident inputs with the cascade of LAPACK dsgesv: early-scale redo, bf16 on fp16 overflow,
+// fp64 fallback (mplu_gesv_device / mplu_gesv_device_nrhs; arguments already checked)
+int gesv_device_impl(mplu_context* c, int n, const double* dA, long long lda, const RhsBlock& b, const mplu_options* opts,
+                     mplu_stats* stats) {
+    CK(cudaSetDevice(c->device));
+    if (opts) c->opts = *opts;
+    const OptionsScope scope(c);
+    resolve_options(c, n);
+    if (stats) memset(stats, 0, sizeof(*stats));
+    c->factored = false;
+    CK(cudaEventRecord(c->ev[0], c->stream));
+    int rc = factor_impl(c, n, dA, lda);
+    if (rc) return rc;
+    CK(cudaEventRecord(c->ev[1], c->stream));
+    rc = solve_rhs(c, dA, lda, b, stats);
+    if (rc == MPLU_E_OVERFLOW && c->used_early_scale) {
+        // the fp16 scale taken from the first block column did not fit a later one: once more with the global scale
+        c->allow_early = false;
+        c->factored = false;
+        rc = factor_impl(c, n, dA, lda);
+        c->allow_early = true;
+        if (rc) return rc;
+        if (stats) memset(stats, 0, sizeof(*stats));
+        rc = solve_rhs(c, dA, lda, b, stats);
+    }
+    if (rc == MPLU_E_OVERFLOW && c->opts.precision == MPLU_FP16 && c->opts.bf16_fallback) {
+        // like dsgesv's fall back to full precision: same algorithm, operand type without the range problem
+        c->opts.precision = MPLU_BF16;
+        c->factored = false;
+        rc = factor_impl(c, n, dA, lda);
+        if (rc) return rc;
+        if (stats) memset(stats, 0, sizeof(*stats));
+        rc = solve_rhs(c, dA, lda, b, stats);
+    }
+    if (stats) {
+        stats->precision_used = c->opts.precision;
+        stats->dsgesv_iter = rc == 0 ? stats->iters : (rc == MPLU_E_OVERFLOW ? -2 : (rc == MPLU_E_NOCONV ? -(stats->iters + 1) : -3));
+    }
+    if ((rc == MPLU_E_OVERFLOW || rc == MPLU_E_ZEROPIVOT || rc == MPLU_E_NOCONV) && c->opts.fp64_fallback)
+        rc = fp64_fallback_solve(c, n, dA, lda, b.nrhs, b.B, b.ldb, b.X, b.ldx, rc, b.berr, stats);  // dsgesv: full-precision factorization and solve
+    CK(cudaEventRecord(c->ev[2], c->stream));
+    CK(cudaEventSynchronize(c->ev[2]));
+    if (stats) {
+        cudaEventElapsedTime(&stats->factor_ms, c->ev[0], c->ev[1]);
+        cudaEventElapsedTime(&stats->solve_ms, c->ev[1], c->ev[2]);
+        cudaEventElapsedTime(&stats->total_ms, c->ev[0], c->ev[2]);
+    }
+    return rc;
+}
+
+// n x ncols column-major copy between host and device (one contiguous copy for a single column)
+cudaError_t copy_columns(double* dst, long long ldd, const double* src, long long lds, int n, int ncols, cudaMemcpyKind kind,
+                         cudaStream_t st) {
+    if (ncols == 1) return cudaMemcpyAsync(dst, src, n * sizeof(double), kind, st);
+    return cudaMemcpy2DAsync(dst, (size_t)ldd * sizeof(double), src, (size_t)lds * sizeof(double), (size_t)n * sizeof(double),
+                             ncols, kind, st);
+}
+
+// factor + solve from host buffers (mplu_gesv_host / mplu_gesv_host_nrhs; arguments already checked): b holds HOST pointers
+int gesv_host_impl(mplu_context* c, int n, const double* hA, long long lda, const RhsBlock& hb, const mplu_options* opts,
+                   mplu_stats* stats) {
+    CK(cudaSetDevice(c->device));
+    const size_t need = (size_t)n * n;
+    if (need > c->dA_cap) {
+        cudaFree(c->dA_stage);
+        c->dA_stage = nullptr; c->dA_cap = 0;
+        CK(cudaMalloc(&c->dA_stage, need * sizeof(double)));
+        c->dA_cap = need;
+    }
+    const size_t vneed = (size_t)n * hb.nrhs;
+    if (vneed > c->dv_cap) {
+        cudaFree(c->db_stage); cudaFree(c->dx_stage);
+        c->db_stage = c->dx_stage = nullptr; c->dv_cap = 0;
+        CK(cudaMalloc(&c->db_stage, vneed * sizeof(double)));
+        CK(cudaMalloc(&c->dx_stage, vneed * sizeof(double)));
+        c->dv_cap = vneed;
+    }
+    const RhsBlock db{hb.nrhs, c->db_stage, n, c->dx_stage, n, hb.berr};  // the staged copies (ld n)
+    cudaStream_t st = c->stream;
+    if (opts) c->opts = *opts;
+    const OptionsScope scope(c);
+    const mplu_options used = c->opts;  // the request: the device path below resolves it again for itself
+    resolve_options(c, n);
+    CK(cudaEventRecord(c->ev[3], st));
+    int rc;
+    float h2d = 0.f;
+    if (c->opts.stream_host && streamed_supported(c, n)) {
+        // block columns are factored as they arrive (factor_streamed); the staged copy of A stays for the residuals
+        if (stats) memset(stats, 0, sizeof(*stats));
+        c->factored = false;
+        CK(cudaStreamWaitEvent(c->copy, c->ev[3], 0));
+        CK(copy_columns(c->db_stage, n, hb.B, hb.ldb, n, hb.nrhs, cudaMemcpyHostToDevice, st));
+        rc = factor_streamed(c, n, hA, lda, c->dA_stage);
+        if (rc) return rc;
+        CK(cudaEventRecord(c->ev[1], st));
+        rc = solve_rhs(c, c->dA_stage, n, db, stats);
+        if (stats) {
+            stats->precision_used = c->opts.precision;
+            stats->dsgesv_iter = rc == 0 ? stats->iters : (rc == MPLU_E_OVERFLOW ? -2 : (rc == MPLU_E_NOCONV ? -(stats->iters + 1) : -3));
+        }
+        if ((rc == MPLU_E_ZEROPIVOT || rc == MPLU_E_NOCONV) && c->opts.fp64_fallback)
+            rc = fp64_fallback_solve(c, n, c->dA_stage, n, db.nrhs, db.B, db.ldb, db.X, db.ldx, rc, db.berr, stats);
+        CK(cudaEventRecord(c->ev[2], st));
+        CK(cudaEventSynchronize(c->ev[2]));
+        cudaEventElapsedTime(&h2d, c->ev[3], c->ev_copy[c->copy_last]);
+        if (stats) {
+            // total = h2d (start .. last byte on the device) + factor (the tail left after it) + solve
+            cudaEventElapsedTime(&stats->factor_ms, c->ev_copy[c->copy_last], c->ev[1]);
+            cudaEventElapsedTime(&stats->solve_ms, c->ev[1], c->ev[2]);
+            stats->total_ms = stats->factor_ms + stats->solve_ms;
+        }
+        if (rc == MPLU_E_OVERFLOW) {
+            // the scale taken from the first block column did not fit a later one: A is resident now, redo the solve
+            // with the global scale (and, if that overflows too, in bf16)
+            const float streamed_ms = h2d + (stats ? stats->total_ms : 0.f);
+            rc = gesv_device_impl(c, n, c->dA_stage, n, db, &used, stats);
+            h2d = streamed_ms;  // everything before the redo counts as transfer time
+        }
+    } else {
+        CK(cudaMemcpy2DAsync(c->dA_stage, (size_t)n * sizeof(double), hA, (size_t)lda * sizeof(double),
+                             (size_t)n * sizeof(double), n, cudaMemcpyHostToDevice, st));
+        CK(copy_columns(c->db_stage, n, hb.B, hb.ldb, n, hb.nrhs, cudaMemcpyHostToDevice, st));
+        rc = gesv_device_impl(c, n, c->dA_stage, n, db, &used, stats);
+        cudaEventElapsedTime(&h2d, c->ev[3], c->ev[0]);
+    }
+    if (rc != 0 && rc != MPLU_E_NOCONV) return rc;
+    CK(cudaEventRecord(c->ev[0], st));
+    CK(copy_columns(hb.X, hb.ldx, c->dx_stage, n, n, hb.nrhs, cudaMemcpyDeviceToHost, st));
+    CK(cudaEventRecord(c->ev[1], st));
+    CK(cudaEventSynchronize(c->ev[1]));
+    if (stats) {
+        float d2h = 0.f;
+        cudaEventElapsedTime(&d2h, c->ev[0], c->ev[1]);
+        stats->h2d_ms = h2d;
+        stats->d2h_ms = d2h;
+        stats->total_ms += h2d + d2h;
+    }
+    return rc;
+}
+
+// the regions spanned by the columns of B and X (first to last element) share an address: X would overwrite B
+bool columns_overlap(const double* B, long long ldb, const double* X, long long ldx, int n, int nrhs) {
+    const double* b1 = B + (long long)(nrhs - 1) * ldb + n;
+    const double* x1 = X + (long long)(nrhs - 1) * ldx + n;
+    return X < b1 && B < x1;
+}
+
+// berr of a one-column call, from the single-vector path's stats
+void single_berr(const mplu_stats* stats, double* berr) {
+    if (berr) berr[0] = backward_error(stats->rnorm_inf, stats->anorm_inf, stats->xnorm_inf, stats->bnorm_inf);
 }
 
 }  // namespace mplu_detail
@@ -1827,129 +2122,47 @@ int mplu_solve_device(mplu_context* c, const double* dA, long long lda, const do
 int mplu_gesv_device(mplu_context* c, int n, const double* dA, long long lda, const double* db, double* dx,
                      const mplu_options* opts, mplu_stats* stats) {
     if (!c || !dA || !db || !dx || n <= 0 || lda < n) return MPLU_E_ARG;
-    CK(cudaSetDevice(c->device));
-    if (opts) c->opts = *opts;
-    const OptionsScope scope(c);
-    resolve_options(c, n);
-    if (stats) memset(stats, 0, sizeof(*stats));
-    c->factored = false;
-    CK(cudaEventRecord(c->ev[0], c->stream));
-    int rc = factor_impl(c, n, dA, lda);
-    if (rc) return rc;
-    CK(cudaEventRecord(c->ev[1], c->stream));
-    rc = solve_impl(c, dA, lda, db, dx, stats);
-    if (rc == MPLU_E_OVERFLOW && c->used_early_scale) {
-        // the fp16 scale taken from the first block column did not fit a later one: once more with the global scale
-        c->allow_early = false;
-        c->factored = false;
-        rc = factor_impl(c, n, dA, lda);
-        c->allow_early = true;
-        if (rc) return rc;
-        if (stats) memset(stats, 0, sizeof(*stats));
-        rc = solve_impl(c, dA, lda, db, dx, stats);
-    }
-    if (rc == MPLU_E_OVERFLOW && c->opts.precision == MPLU_FP16 && c->opts.bf16_fallback) {
-        // like dsgesv's fall back to full precision: same algorithm, operand type without the range problem
-        c->opts.precision = MPLU_BF16;
-        c->factored = false;
-        rc = factor_impl(c, n, dA, lda);
-        if (rc) return rc;
-        if (stats) memset(stats, 0, sizeof(*stats));
-        rc = solve_impl(c, dA, lda, db, dx, stats);
-    }
-    if (stats) {
-        stats->precision_used = c->opts.precision;
-        stats->dsgesv_iter = rc == 0 ? stats->iters : (rc == MPLU_E_OVERFLOW ? -2 : (rc == MPLU_E_NOCONV ? -(stats->iters + 1) : -3));
-    }
-    if ((rc == MPLU_E_OVERFLOW || rc == MPLU_E_ZEROPIVOT || rc == MPLU_E_NOCONV) && c->opts.fp64_fallback)
-        rc = fp64_fallback_solve(c, n, dA, lda, db, dx, rc, stats);  // dsgesv: full-precision factorization and solve
-    CK(cudaEventRecord(c->ev[2], c->stream));
-    CK(cudaEventSynchronize(c->ev[2]));
-    if (stats) {
-        cudaEventElapsedTime(&stats->factor_ms, c->ev[0], c->ev[1]);
-        cudaEventElapsedTime(&stats->solve_ms, c->ev[1], c->ev[2]);
-        cudaEventElapsedTime(&stats->total_ms, c->ev[0], c->ev[2]);
-    }
-    return rc;
+    return gesv_device_impl(c, n, dA, lda, RhsBlock{1, db, n, dx, n, nullptr}, opts, stats);
 }
 
 int mplu_gesv_host(mplu_context* c, int n, const double* hA, long long lda, const double* hb, double* hx,
                    const mplu_options* opts, mplu_stats* stats) {
     if (!c || !hA || !hb || !hx || n <= 0 || lda < n) return MPLU_E_ARG;
+    return gesv_host_impl(c, n, hA, lda, RhsBlock{1, hb, n, hx, n, nullptr}, opts, stats);
+}
+
+int mplu_solve_device_nrhs(mplu_context* c, int nrhs, const double* dA, long long lda, const double* dB, long long ldb,
+                           double* dX, long long ldx, double* berr, mplu_stats* stats) {
+    if (!c || !dA || !dB || !dX || nrhs < 1 || lda < c->n || ldb < c->n || ldx < c->n) return MPLU_E_ARG;
+    if (columns_overlap(dB, ldb, dX, ldx, c->n, nrhs)) return MPLU_E_ARG;
     CK(cudaSetDevice(c->device));
-    const size_t need = (size_t)n * n;
-    if (need > c->dA_cap) {
-        cudaFree(c->dA_stage);
-        c->dA_stage = nullptr; c->dA_cap = 0;
-        CK(cudaMalloc(&c->dA_stage, need * sizeof(double)));
-        c->dA_cap = need;
-    }
-    if ((size_t)n > c->dv_cap) {
-        cudaFree(c->db_stage); cudaFree(c->dx_stage);
-        c->db_stage = c->dx_stage = nullptr; c->dv_cap = 0;
-        CK(cudaMalloc(&c->db_stage, n * sizeof(double)));
-        CK(cudaMalloc(&c->dx_stage, n * sizeof(double)));
-        c->dv_cap = n;
-    }
-    cudaStream_t st = c->stream;
-    if (opts) c->opts = *opts;
-    const OptionsScope scope(c);
-    const mplu_options used = c->opts;  // the request: the device path below resolves it again for itself
-    resolve_options(c, n);
-    CK(cudaEventRecord(c->ev[3], st));
-    int rc;
-    float h2d = 0.f;
-    if (c->opts.stream_host && streamed_supported(c, n)) {
-        // block columns are factored as they arrive (factor_streamed); the staged copy of A stays for the residuals
-        if (stats) memset(stats, 0, sizeof(*stats));
-        c->factored = false;
-        CK(cudaStreamWaitEvent(c->copy, c->ev[3], 0));
-        CK(cudaMemcpyAsync(c->db_stage, hb, n * sizeof(double), cudaMemcpyHostToDevice, st));
-        rc = factor_streamed(c, n, hA, lda, c->dA_stage);
-        if (rc) return rc;
-        CK(cudaEventRecord(c->ev[1], st));
-        rc = solve_impl(c, c->dA_stage, n, c->db_stage, c->dx_stage, stats);
-        if (stats) {
-            stats->precision_used = c->opts.precision;
-            stats->dsgesv_iter = rc == 0 ? stats->iters : (rc == MPLU_E_OVERFLOW ? -2 : (rc == MPLU_E_NOCONV ? -(stats->iters + 1) : -3));
-        }
-        if ((rc == MPLU_E_ZEROPIVOT || rc == MPLU_E_NOCONV) && c->opts.fp64_fallback)
-            rc = fp64_fallback_solve(c, n, c->dA_stage, n, c->db_stage, c->dx_stage, rc, stats);
-        CK(cudaEventRecord(c->ev[2], st));
-        CK(cudaEventSynchronize(c->ev[2]));
-        cudaEventElapsedTime(&h2d, c->ev[3], c->ev_copy[c->copy_last]);
-        if (stats) {
-            // total = h2d (start .. last byte on the device) + factor (the tail left after it) + solve
-            cudaEventElapsedTime(&stats->factor_ms, c->ev_copy[c->copy_last], c->ev[1]);
-            cudaEventElapsedTime(&stats->solve_ms, c->ev[1], c->ev[2]);
-            stats->total_ms = stats->factor_ms + stats->solve_ms;
-        }
-        if (rc == MPLU_E_OVERFLOW) {
-            // the scale taken from the first block column did not fit a later one: A is resident now, redo the solve
-            // with the global scale (and, if that overflows too, in bf16)
-            const float streamed_ms = h2d + (stats ? stats->total_ms : 0.f);
-            rc = mplu_gesv_device(c, n, c->dA_stage, n, c->db_stage, c->dx_stage, &used, stats);
-            h2d = streamed_ms;  // everything before the redo counts as transfer time
-        }
-    } else {
-        CK(cudaMemcpy2DAsync(c->dA_stage, (size_t)n * sizeof(double), hA, (size_t)lda * sizeof(double),
-                             (size_t)n * sizeof(double), n, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(c->db_stage, hb, n * sizeof(double), cudaMemcpyHostToDevice, st));
-        rc = mplu_gesv_device(c, n, c->dA_stage, n, c->db_stage, c->dx_stage, &used, stats);
-        cudaEventElapsedTime(&h2d, c->ev[3], c->ev[0]);
-    }
-    if (rc != 0 && rc != MPLU_E_NOCONV) return rc;
-    CK(cudaEventRecord(c->ev[0], st));
-    CK(cudaMemcpyAsync(hx, c->dx_stage, n * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CK(cudaEventRecord(c->ev[1], st));
-    CK(cudaEventSynchronize(c->ev[1]));
-    if (stats) {
-        float d2h = 0.f;
-        cudaEventElapsedTime(&d2h, c->ev[0], c->ev[1]);
-        stats->h2d_ms = h2d;
-        stats->d2h_ms = d2h;
-        stats->total_ms += h2d + d2h;
-    }
+    mplu_stats local;
+    if (!stats) stats = &local;
+    memset(stats, 0, sizeof(*stats));
+    const int rc = solve_rhs(c, dA, lda, RhsBlock{nrhs, dB, ldb, dX, ldx, berr}, stats);
+    if (nrhs == 1) single_berr(stats, berr);
+    return rc;
+}
+
+int mplu_gesv_device_nrhs(mplu_context* c, int n, int nrhs, const double* dA, long long lda, const double* dB, long long ldb,
+                          double* dX, long long ldx, const mplu_options* opts, double* berr, mplu_stats* stats) {
+    if (!c || !dA || !dB || !dX || n <= 0 || nrhs < 1 || lda < n || ldb < n || ldx < n) return MPLU_E_ARG;
+    if (columns_overlap(dB, ldb, dX, ldx, n, nrhs)) return MPLU_E_ARG;
+    mplu_stats local;
+    if (!stats) stats = &local;
+    const int rc = gesv_device_impl(c, n, dA, lda, RhsBlock{nrhs, dB, ldb, dX, ldx, berr}, opts, stats);
+    if (nrhs == 1) single_berr(stats, berr);
+    return rc;
+}
+
+int mplu_gesv_host_nrhs(mplu_context* c, int n, int nrhs, const double* hA, long long lda, const double* hB, long long ldb,
+                        double* hX, long long ldx, const mplu_options* opts, double* berr, mplu_stats* stats) {
+    if (!c || !hA || !hB || !hX || n <= 0 || nrhs < 1 || lda < n || ldb < n || ldx < n) return MPLU_E_ARG;
+    if (columns_overlap(hB, ldb, hX, ldx, n, nrhs)) return MPLU_E_ARG;
+    mplu_stats local;
+    if (!stats) stats = &local;
+    const int rc = gesv_host_impl(c, n, hA, lda, RhsBlock{nrhs, hB, ldb, hX, ldx, berr}, opts, stats);
+    if (nrhs == 1) single_berr(stats, berr);
     return rc;
 }
 

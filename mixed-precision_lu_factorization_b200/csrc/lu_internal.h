@@ -46,6 +46,12 @@ struct mplu_context {
     double* norms = nullptr;  // [0] ||r||, [1] ||x||
     float* y = nullptr;       // 2*npad
     int nchunk = 64;
+    // several right-hand sides (mplu_*_nrhs): allocated on the first call with nrhs > 1, freed with the other work arrays
+    double* rb_R = nullptr;        // n x nrhs residual block (ld n)
+    double* rb_partial = nullptr;  // kResidualChunks * kResidualBlock * n
+    double* rb_norms = nullptr;    // per column ||r||, ||x||, then ||b|| per column
+    float* rb_y = nullptr;         // 2 * npad * kSolveBlock (the batched solve's fp32 work blocks)
+    int rb_cap_n = 0, rb_cap_npad = 0, rb_cap_nrhs = 0;
     // GMRES-IR workspace (gmres.cu)
     double* gm_V = nullptr; double* gm_w = nullptr; double* gm_h = nullptr; double* gm_zero = nullptr;
     int gm_cap_n = 0, gm_cap_m = 0;
@@ -181,11 +187,15 @@ int run_gemm_pair(mplu_context* c, const Lane& ln, const GemmCall& g0, const Gem
 // c->Linv32 / c->Uinv32.  Everything is enqueued on `st`.
 int getrf_resident_tile(mplu_context* c, cudaStream_t st, int w);
 int ensure_work(mplu_context* c, int n);
-// GMRES-IR: solve A d = c->r by GMRES preconditioned with the stored factors, x += d (gmres.cu)
-int gmres_correction(mplu_context* c, const double* dA, long long lda, double* dx, int* inner);
+// GMRES-IR: solve A d = r (n doubles on the device) by GMRES preconditioned with the stored factors, x += d (gmres.cu)
+int gmres_correction(mplu_context* c, const double* dA, long long lda, const double* r, double* dx, int* inner);
 // dsgesv-style full-precision redo of a solve the low-precision factors could not deliver (fp64_fallback.cu); `why` is the
-// MPLU_E_* code the mixed-precision path ended with
-int fp64_fallback_solve(mplu_context* c, int n, const double* dA, long long lda, const double* db, double* dx, int why,
-                        mplu_stats* stats);
+// MPLU_E_* code the mixed-precision path ended with.  nrhs column-major right-hand sides (B, ldb) and solutions (X, ldx):
+// one fp64 factorization, then every column is solved and refined on its own; berr (host, may be null) receives each
+// column's backward error, stats the worst column's figures
+int fp64_fallback_solve(mplu_context* c, int n, const double* dA, long long lda, int nrhs, const double* dB, long long ldb,
+                        double* dX, long long ldx, int why, double* berr, mplu_stats* stats);
+// the per-column backward error ||r|| / (||A|| ||x|| + ||b||) (0 for r = 0: a zero column is solved exactly)
+inline double backward_error(double rn, double an, double xn, double bn) { return rn == 0.0 ? 0.0 : rn / (an * xn + bn); }
 
 }  // namespace mplu_detail

@@ -122,14 +122,6 @@ __global__ void local_first_touch_kernel(const double* __restrict__ A, long long
     if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<int*>(amax), __float_as_int(lmax));
 }
 
-__global__ void max_abs_f64_kernel(const double* v, int n, double* out) {
-    double m = 0.0;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) m = fmax(m, fabs(v[i]));
-    for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
-    if ((threadIdx.x & 31) == 0)
-        atomicMax(reinterpret_cast<unsigned long long*>(out), (unsigned long long)__double_as_longlong(m));
-}
-
 // y_full[global row] += sum_{local cols in chunk} A_loc(row, c) * x[global col(c)]   (fp64, HBM-bound: 8 B / element)
 // grid (ceil(mloc/256), chunks); thread = 2 consecutive local rows (mloc, nb even).
 __global__ void __launch_bounds__(128)
@@ -398,8 +390,8 @@ int alloc_rank_work(mplu_dist* d, DRank& r) {
     CK(cudaMalloc(&r.r, n * sizeof(double)));
     CK(cudaMalloc(&r.ax, n * sizeof(double)));
     CK(cudaMalloc(&r.rowsum, n * sizeof(double)));
-    CK(cudaMalloc(&r.norms, 2 * sizeof(double)));
-    CK(cudaMalloc(&r.anorm, 2 * sizeof(double)));
+    CK(cudaMalloc(&r.norms, 3 * sizeof(double)));  // ||r||, ||x||, ||b||: RefineOps::norms for one column
+    CK(cudaMalloc(&r.anorm, sizeof(double)));
     CK(cudaMalloc(&r.yv, n * sizeof(float)));
     CK(cudaMalloc(&r.xv, n * sizeof(float)));
     CK(cudaMalloc(&r.part, 2 * (size_t)n * sizeof(float)));
@@ -541,8 +533,7 @@ int enqueue_dist_factorization(mplu_dist* d) {
     CKI(allreduce(d, 2, 1, [](DRank& r) { return (void*)r.ctx->amax; }, chain_of));
     CKI(allreduce(d, 1, (size_t)d->n, [](DRank& r) { return (void*)r.rowsum; }, chain_of));
     for (auto& r : d->ranks) {
-        CK(cudaMemsetAsync(r.anorm, 0, 2 * sizeof(double), r.chain));
-        max_abs_f64_kernel<<<64, 256, 0, r.chain>>>(r.rowsum, d->n, r.anorm);
+        CKI(launch_column_absmax(r.rowsum, d->n, d->n, 1, r.anorm, r.chain));
         CKI(launch_scales(r.ctx->amax, r.ctx->scales, d->opts.a_exp, d->opts.l_exp, bf16, r.chain));
         CK(cudaMemcpyAsync(r.dctx->scales, r.ctx->scales, SC_COUNT * sizeof(float), cudaMemcpyDeviceToDevice, r.chain));
         if (r.mloc > 0 && r.nloc > 0)
@@ -1251,39 +1242,33 @@ int mplu_dist_gesv(mplu_dist* d, int n, int nb, const double* const* dA, const l
     CKI(enqueue_dist_factorization(d));
     CK(cudaEventRecord(d->ev1, r0.chain));
 
-    // ||b||_inf, first solve x = (LU)^-1 b
-    for (size_t i = 0; i < d->ranks.size(); ++i) {
-        DRank& r = d->ranks[i];
-        max_abs_f64_kernel<<<64, 256, 0, r.chain>>>(bv[i], n, r.anorm + 1);
-    }
-    CKI(enqueue_lu_solve(d, bv));
-    for (size_t i = 0; i < d->ranks.size(); ++i)
-        apply_correction_kernel<<<(n + 255) / 256, 256, 0, d->ranks[i].chain>>>(d->ranks[i].xv, xv[i], n, 0);
-
-    double h_norms[2] = {0, 0}, h_an[2] = {0, 0};
-    const double eps = 2.220446049250313e-16 / 2.0;
-    int iters = 0, converged = 0;
-    double first_be = -1.0;
-    const int max_iters = d->opts.max_iters > 0 ? d->opts.max_iters : 30;
-    std::vector<const double*> xc(xv.begin(), xv.end());
-    for (;;) {
-        CKI(enqueue_residual(d, bv, xv));
-        // every process takes the decision from its own (identical) copy of the norms
-        CK(cudaMemcpyAsync(h_norms, r0.norms, 2 * sizeof(double), cudaMemcpyDeviceToHost, r0.chain));
-        if (first_be < 0) CK(cudaMemcpyAsync(h_an, r0.anorm, 2 * sizeof(double), cudaMemcpyDeviceToHost, r0.chain));
-        for (auto& r : d->ranks) CK(cudaStreamSynchronize(r.chain));
-        const double be = h_norms[0] / (h_an[0] * h_norms[1] + h_an[1]);
-        if (first_be < 0) first_be = be;
-        const double thresh = d->opts.tol > 0 ? d->opts.tol * h_an[0] * h_norms[1]
-                                               : h_norms[1] * h_an[0] * eps * std::sqrt((double)n);
-        if (!(h_norms[0] == h_norms[0])) break;
-        if (h_norms[0] <= thresh) { converged = 1; break; }
-        if (iters >= max_iters) break;
+    // ||b||_inf and the first solve x = (LU)^-1 b, then dsgesv's refinement.  Every process takes the decision from its
+    // own (identical) copy of the norms.
+    RefineOps ops;
+    ops.norms = r0.norms;
+    ops.anorm = r0.anorm;
+    ops.st = r0.chain;
+    ops.first_solve = [&]() -> int {
+        for (size_t i = 0; i < d->ranks.size(); ++i)
+            CKI(launch_column_absmax(bv[i], n, n, 1, d->ranks[i].norms + 2, d->ranks[i].chain));
+        CKI(enqueue_lu_solve(d, bv));
+        for (size_t i = 0; i < d->ranks.size(); ++i)
+            apply_correction_kernel<<<(n + 255) / 256, 256, 0, d->ranks[i].chain>>>(d->ranks[i].xv, xv[i], n, 0);
+        return 0;
+    };
+    ops.residual = [&](bool*) { return enqueue_residual(d, bv, xv); };
+    ops.correct = [&](int*) -> int {
         CKI(enqueue_lu_solve(d, rv));
         for (size_t i = 0; i < d->ranks.size(); ++i)
             apply_correction_kernel<<<(n + 255) / 256, 256, 0, d->ranks[i].chain>>>(d->ranks[i].xv, xv[i], n, 1);
-        ++iters;
-    }
+        return 0;
+    };
+    ops.wait = [&]() -> int {
+        for (auto& r : d->ranks) CK(cudaStreamSynchronize(r.chain));
+        return 0;
+    };
+    RefineResult res;
+    CKI(refine(ops, n, 1, d->opts.max_iters, d->opts.tol, &res));
     CK(cudaEventRecord(d->ev2, r0.chain));
     CK(cudaEventSynchronize(d->ev2));
     int h_status = 0;
@@ -1293,17 +1278,9 @@ int mplu_dist_gesv(mplu_dist* d, int n, int nb, const double* const* dA, const l
         CK(cudaMemcpy(&s2, r.dctx->status, sizeof(int), cudaMemcpyDeviceToHost));
         h_status |= s1 | s2;
     }
+    refine_stats(res, n, nullptr, stats);
     if (stats) {
-        stats->n = n;
-        stats->iters = iters;
-        stats->converged = converged;
         stats->status_bits = h_status;
-        stats->anorm_inf = h_an[0];
-        stats->bnorm_inf = h_an[1];
-        stats->xnorm_inf = h_norms[1];
-        stats->rnorm_inf = h_norms[0];
-        stats->backward_error = h_norms[0] / (h_an[0] * h_norms[1] + h_an[1]);
-        stats->first_backward_error = first_be;
         stats->gemm_launches = d->gemm_launches;
         stats->kernel_launches = d->kernel_launches;
         stats->trailing_launches = d->trail_count;
@@ -1319,10 +1296,7 @@ int mplu_dist_gesv(mplu_dist* d, int n, int nb, const double* const* dA, const l
         cudaEventElapsedTime(&stats->solve_ms, d->ev1, d->ev2);
         cudaEventElapsedTime(&stats->total_ms, d->ev0, d->ev2);
     }
-    if (converged) return 0;
-    if (h_status & 1) return MPLU_E_OVERFLOW;
-    if (h_status & 2) return MPLU_E_ZEROPIVOT;
-    return MPLU_E_NOCONV;
+    return refine_rc(res.converged, h_status);
 }
 
 // Same solve from HOST buffers (pinned or pageable): hA[i] = local block-cyclic fp64 tiles of logical rank i (host,

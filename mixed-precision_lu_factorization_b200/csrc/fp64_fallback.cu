@@ -9,8 +9,7 @@
 // A rare path: written for clarity, not speed (one launch per 128-block of each triangular sweep).
 #include "lu_internal.h"
 
-#include <cmath>
-#include <cstring>
+#include <algorithm>
 
 namespace mplu_detail {
 
@@ -122,66 +121,50 @@ int fp64_fallback_solve(mplu_context* c, int n, const double* dA, long long lda,
             CK(cudaStreamSynchronize(st));
         }
         CK(mpf_device(LU, n, 32, ipiv));
-        // every column is solved and refined on its own; stats report the column with the largest backward error
-        int all_converged = 1, max_iters_seen = 0;
-        double worst = -1.0, worst_first = -1.0;
+        // every column is solved and refined on its own, at most 5 corrections each; stats report the worst column
+        const double* db = nullptr;
+        double* dx = nullptr;
+        bool first = true;
+        RefineOps ops;
+        ops.norms = c->norms;
+        ops.anorm = c->anorm;
+        ops.st = st;
+        ops.first_solve = [&]() -> int {
+            CKI(mplu::launch_column_absmax(db, n, n, 1, c->norms + 2, st));
+            return lu_solve_fp64(LU, n, ipiv, db, dx, tmp, st);
+        };
+        ops.residual = [&](bool* formed_anorm) -> int {
+            // the row sums of |A| ride along in the first pass (the low-precision path may not have got that far)
+            *formed_anorm = first;
+            first = false;
+            return mplu::launch_residual(dA, lda, n, dx, db, c->r, c->partial, c->nchunk, c->norms, st,
+                                         *formed_anorm ? c->rowsum_part : nullptr, *formed_anorm ? c->anorm : nullptr);
+        };
+        ops.correct = [&](int*) -> int {
+            CKI(lu_solve_fp64(LU, n, ipiv, c->r, d, tmp, st));
+            axpy_kernel<<<(n + 255) / 256, 256, 0, st>>>(dx, d, n);
+            return 0;
+        };
+        ops.wait = [&]() -> int { return (int)cudaStreamSynchronize(st); };
+        RefineResult all;
+        all.converged = 1;
         for (int col = 0; col < nrhs; ++col) {
-            const double* db = dB + (long long)col * ldb;
-            double* dx = dX + (long long)col * ldx;
-            CKI(lu_solve_fp64(LU, n, ipiv, db, dx, tmp, st));
-            const double eps = 2.220446049250313e-16 / 2.0;
-            double h_norms[2] = {0, 0}, h_an[2] = {0, 0};
-            int iters = 0, converged = 0;
-            double first_be = -1.0;
-            CK(cudaMemsetAsync(c->anorm + 1, 0, sizeof(double), st));
-            for (;;) {
-                // the row sums of |A| ride along in the first pass (the low-precision path may not have got that far)
-                const bool with_anorm = first_be < 0;
-                CKI(mplu::launch_residual(dA, lda, n, dx, db, c->r, c->partial, c->nchunk, c->norms, st, with_anorm ? c->rowsum_part : nullptr,
-                                          with_anorm ? c->anorm : nullptr));
-                CK(cudaMemcpyAsync(h_norms, c->norms, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-                if (with_anorm) CK(cudaMemcpyAsync(h_an, c->anorm, sizeof(double), cudaMemcpyDeviceToHost, st));
-                CK(cudaStreamSynchronize(st));
-                if (with_anorm) {  // ||b||_inf on the host side of the residual: r = b when x = 0 is not available; take it from b directly
-                    std::vector<double> hb(n);
-                    CK(cudaMemcpy(hb.data(), db, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost));
-                    for (double v : hb) h_an[1] = std::fmax(h_an[1], std::fabs(v));
-                }
-                const double be = h_norms[0] / (h_an[0] * h_norms[1] + h_an[1]);
-                if (first_be < 0) first_be = be;
-                const double thresh = c->opts.tol > 0 ? c->opts.tol * h_an[0] * h_norms[1] : h_norms[1] * h_an[0] * eps * std::sqrt((double)n);
-                if (!(h_norms[0] == h_norms[0])) break;
-                if (h_norms[0] <= thresh) { converged = 1; break; }
-                if (iters >= 5) break;
-                CKI(lu_solve_fp64(LU, n, ipiv, c->r, d, tmp, st));
-                axpy_kernel<<<(n + 255) / 256, 256, 0, st>>>(dx, d, n);
-                ++iters;
-            }
-            const double be_col = backward_error(h_norms[0], h_an[0], h_norms[1], h_an[1]);
-            if (berr) berr[col] = be_col;
-            all_converged &= converged;
-            max_iters_seen = iters > max_iters_seen ? iters : max_iters_seen;
-            worst_first = (col == 0 || first_be > worst_first) ? first_be : worst_first;
-            const bool is_worst = col == 0 || be_col > worst || be_col != be_col;
-            if (is_worst) worst = be_col;
-            if (stats && is_worst) {
-                stats->n = n;
-                stats->anorm_inf = h_an[0];
-                stats->bnorm_inf = h_an[1];
-                stats->xnorm_inf = h_norms[1];
-                stats->rnorm_inf = h_norms[0];
-                stats->backward_error = nrhs == 1 ? h_norms[0] / (h_an[0] * h_norms[1] + h_an[1]) : be_col;
-            }
+            db = dB + (long long)col * ldb;
+            dx = dX + (long long)col * ldx;
+            first = true;
+            RefineResult one;
+            CKI(refine(ops, n, 1, 5, c->opts.tol, &one));
+            all.col.push_back(one.col[0]);
+            all.anorm = one.anorm;
+            all.iters = std::max(all.iters, one.iters);
+            all.converged &= one.converged;
         }
+        refine_stats(all, n, berr, stats);
         if (stats) {
-            stats->iters = max_iters_seen;
-            stats->converged = all_converged;
-            stats->first_backward_error = worst_first;
             stats->fp64_fallback = 1;
-            const int max_iters = c->opts.max_iters > 0 ? c->opts.max_iters : 30;
-            stats->dsgesv_iter = why == MPLU_E_OVERFLOW ? -2 : (why == MPLU_E_NOCONV ? -(max_iters + 1) : -3);
+            stats->dsgesv_iter = dsgesv_iter(why, c->opts.max_iters > 0 ? c->opts.max_iters : 30);
         }
-        return all_converged ? 0 : MPLU_E_NOCONV;
+        return refine_rc(all.converged, 0);
     };
     rc = body();
     cudaStreamSynchronize(st);

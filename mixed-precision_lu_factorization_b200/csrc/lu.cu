@@ -1620,14 +1620,6 @@ int factor_streamed(mplu_context* c, int n, const double* hA, long long lda, dou
     return 0;
 }
 
-__global__ void absmax_kernel(const double* v, int n, double* out) {
-    double m = 0.0;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) m = fmax(m, fabs(v[i]));
-    for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
-    if ((threadIdx.x & 31) == 0)
-        atomicMax(reinterpret_cast<unsigned long long*>(out), (unsigned long long)__double_as_longlong(m));
-}
-
 __global__ void widen_kernel(const float* __restrict__ W, long long ldw, int n, double* __restrict__ out,
                              long long ldo) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1635,195 +1627,77 @@ __global__ void widen_kernel(const float* __restrict__ W, long long ldw, int n, 
     for (int c = blockIdx.y; c < n; c += gridDim.y) out[r + (long long)c * ldo] = (double)W[r + (long long)c * ldw];
 }
 
-int solve_impl(mplu_context* c, const double* dA, long long lda, const double* db, double* dx, mplu_stats* stats) {
-    if (!c->factored) return MPLU_E_NOTFACTORED;
-    const int n = c->n, npad = c->npad;
-    const long long ld = npad;
-    cudaStream_t st = c->stream;
-    const int solve_launches = 1;
-
-    CK(cudaMemsetAsync(c->anorm + 1, 0, sizeof(double), st));
-    absmax_kernel<<<64, 256, 0, st>>>(db, n, c->anorm + 1);
-    // first solve: x = (LU)^-1 b
-    CKI(launch_lu_solve(c->W, ld, n, npad, c->Linv32, c->Uinv32, db, c->y, dx, nullptr, c->ready, st));
-    c->kernel_launches += solve_launches + 1;
-
-    double h_norms[2] = {0, 0}, h_an[2] = {0, 0};
+int refine(const RefineOps& ops, int n, int k, int max_iters, double tol, RefineResult* res) {
     const double eps = 2.220446049250313e-16 / 2.0;  // LAPACK dlamch('E')
-    int iters = 0, converged = 0, gmres_iters = 0;
-    double first_be = -1.0;
-    const int max_iters = c->opts.max_iters > 0 ? c->opts.max_iters : 30;
-    for (;;) {
-        // lazy first touch: ||A||_inf rides in the first residual pass (it streams all of A anyway)
-        const bool with_anorm = c->anorm_pending;
-        CKI(launch_residual(dA, lda, n, dx, db, c->r, c->partial, c->nchunk, c->norms, st, with_anorm ? c->rowsum_part : nullptr,
-                            with_anorm ? c->anorm : nullptr));
-        c->anorm_pending = false;
-        c->kernel_launches += 2;
-        CK(cudaMemcpyAsync(h_norms, c->norms, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-        if (first_be < 0 || with_anorm) CK(cudaMemcpyAsync(h_an, c->anorm, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        const double be = h_norms[0] / (h_an[0] * h_norms[1] + h_an[1]);
-        if (first_be < 0) first_be = be;
-        double thresh;
-        if (c->opts.tol > 0) thresh = c->opts.tol * h_an[0] * h_norms[1];
-        else thresh = h_norms[1] * h_an[0] * eps * std::sqrt((double)n);
-        if (!(h_norms[0] == h_norms[0])) break;  // NaN: give up
-        if (h_norms[0] <= thresh) { converged = 1; break; }
-        if (iters >= max_iters) break;
-        if (c->opts.refinement == MPLU_REFINE_GMRES) {
-            int inner = 0;
-            CKI(gmres_correction(c, dA, lda, c->r, dx, &inner));
-            gmres_iters += inner;
-        } else {
-            CKI(launch_lu_solve(c->W, ld, n, npad, c->Linv32, c->Uinv32, c->r, c->y, nullptr, dx, c->ready, st));
-            c->kernel_launches += solve_launches;
+    if (max_iters <= 0) max_iters = 30;
+    res->col.assign(k, RefineColumn{});
+    std::vector<double> h(3 * (size_t)k);
+    CKI(ops.first_solve());
+    for (bool first = true;; first = false) {
+        bool formed_anorm = false;
+        CKI(ops.residual(&formed_anorm));
+        CK(cudaMemcpyAsync(h.data(), ops.norms, h.size() * sizeof(double), cudaMemcpyDeviceToHost, ops.st));
+        if (first || formed_anorm) CK(cudaMemcpyAsync(&res->anorm, ops.anorm, sizeof(double), cudaMemcpyDeviceToHost, ops.st));
+        CKI(ops.wait());
+        const double an = res->anorm;
+        bool all = true, nan = false;
+        for (int j = 0; j < k; ++j) {
+            RefineColumn& cj = res->col[j];
+            cj.rnorm = h[2 * j];
+            cj.xnorm = h[2 * j + 1];
+            cj.bnorm = h[2 * k + j];
+            cj.berr = backward_error(cj.rnorm, an, cj.xnorm, cj.bnorm);
+            if (first) cj.first_berr = cj.berr;
+            const double thresh = tol > 0 ? tol * an * cj.xnorm : cj.xnorm * an * eps * std::sqrt((double)n);
+            if (!(cj.rnorm == cj.rnorm)) nan = true;
+            if (!(cj.rnorm <= thresh)) all = false;
         }
-        ++iters;
+        if (nan) break;  // NaN: give up
+        if (all) { res->converged = 1; break; }
+        if (res->iters >= max_iters) break;
+        int steps = 0;
+        CKI(ops.correct(&steps));
+        res->gmres_iters += steps;
+        ++res->iters;
     }
-    int h_status = 0;
-    CK(cudaMemcpy(&h_status, c->status, sizeof(int), cudaMemcpyDeviceToHost));
-    if (stats) {
-        stats->n = n;
-        stats->iters = iters;
-        stats->converged = converged;
-        stats->status_bits = h_status;
-        stats->anorm_inf = h_an[0];
-        stats->bnorm_inf = h_an[1];
-        stats->xnorm_inf = h_norms[1];
-        stats->rnorm_inf = h_norms[0];
-        stats->backward_error = h_norms[0] / (h_an[0] * h_norms[1] + h_an[1]);
-        stats->first_backward_error = first_be;
-        stats->gemm_launches = c->gemm_launches;
-        stats->kernel_launches = c->kernel_launches;
-        stats->trailing_launches = c->trail_count;
-        stats->trailing_flops = c->trail_flops;
-        stats->trailing_bytes = c->trail_bytes;
-        stats->gmres_iters = gmres_iters;
-        float tms = 0.f;
-        for (int i = 0; i < c->trail_count; ++i) {
-            float ms = 0.f;
-            if (cudaEventElapsedTime(&ms, c->trail_ev[2 * i], c->trail_ev[2 * i + 1]) == cudaSuccess) tms += ms;
-        }
-        stats->trailing_ms = tms;
+    return 0;
+}
+
+void refine_stats(const RefineResult& res, int n, double* berr, mplu_stats* stats) {
+    const int k = (int)res.col.size();
+    if (berr)
+        for (int j = 0; j < k; ++j) berr[j] = res.col[j].berr;
+    if (!stats) return;
+    int w = 0;  // the worst column (a NaN is worse than anything)
+    for (int j = 1; j < k; ++j) {
+        const double bj = res.col[j].berr, bw = res.col[w].berr;
+        if (bj > bw || (bj != bj && bw == bw)) w = j;
     }
+    stats->n = n;
+    stats->iters = res.iters;
+    stats->converged = res.converged;
+    stats->anorm_inf = res.anorm;
+    stats->bnorm_inf = res.col[w].bnorm;
+    stats->xnorm_inf = res.col[w].xnorm;
+    stats->rnorm_inf = res.col[w].rnorm;
+    stats->backward_error = res.col[w].berr;
+    stats->first_backward_error = std::max_element(res.col.begin(), res.col.end(), [](const RefineColumn& a, const RefineColumn& b) {
+        return a.first_berr < b.first_berr;
+    })->first_berr;
+}
+
+int refine_rc(int converged, int status_bits) {
     if (converged) return 0;
-    if (h_status & 1) return MPLU_E_OVERFLOW;
-    if (h_status & 2) return MPLU_E_ZEROPIVOT;
+    if (status_bits & 1) return MPLU_E_OVERFLOW;
+    if (status_bits & 2) return MPLU_E_ZEROPIVOT;
     return MPLU_E_NOCONV;
 }
 
-// solve_impl for nrhs > 1 columns: LAPACK dsgesv's refinement over a block.  X0 = (LU)^-1 B, then every column is refined
-// until all of them meet solve_impl's stopping rule (or max_iters): the columns share the iteration count and nothing
-// else.  A and the factors are streamed once per block of kResidualBlock / kSolveBlock columns.  GMRES refinement runs
-// gmres_correction column by column (not batched).
-int solve_nrhs_impl(mplu_context* c, const double* dA, long long lda, int nrhs, const double* dB, long long ldb, double* dX,
-                    long long ldx, double* berr, mplu_stats* stats) {
-    if (!c->factored) return MPLU_E_NOTFACTORED;
-    const int n = c->n, npad = c->npad;
-    const long long ld = npad;
-    cudaStream_t st = c->stream;
-    CKI(ensure_rhs_work(c, nrhs));
-    double* norms = c->rb_norms;               // [2j] ||r_j||_inf, [2j+1] ||x_j||_inf
-    double* bnorms = c->rb_norms + 2 * nrhs;   // [j] ||b_j||_inf
-    CKI(launch_column_absmax(dB, ldb, n, nrhs, bnorms, st));
-    c->kernel_launches += 1;
-    // D = (LU)^-1 rhs for all columns, kSolveBlock at a time: D -> d_out, or x_accum += D
-    auto solve_blocks = [&](const double* rhs, long long ldr, double* d_out, double* x_accum) -> int {
-        for (int j0 = 0; j0 < nrhs; j0 += kSolveBlock) {
-            const int kc = std::min(kSolveBlock, nrhs - j0);
-            CKI(launch_lu_solve_block(c->W, ld, n, npad, c->Linv32, c->Uinv32, rhs + (long long)j0 * ldr, ldr, kc, c->rb_y,
-                                      d_out ? d_out + (long long)j0 * ldx : nullptr, ldx,
-                                      x_accum ? x_accum + (long long)j0 * ldx : nullptr, ldx, c->ready, st));
-            c->kernel_launches += 2;
-        }
-        return 0;
-    };
-    CKI(solve_blocks(dB, ldb, dX, nullptr));
-
-    std::vector<double> h_norms(3 * (size_t)nrhs), be(nrhs), first_be(nrhs);
-    double anorm = 0.0;
-    const double eps = 2.220446049250313e-16 / 2.0;  // LAPACK dlamch('E')
-    int iters = 0, converged = 0, gmres_iters = 0;
-    bool first_pass = true;
-    const int max_iters = c->opts.max_iters > 0 ? c->opts.max_iters : 30;
-    for (;;) {
-        // lazy first touch: ||A||_inf rides in the first residual pass of the first column block
-        const bool with_anorm = c->anorm_pending;
-        for (int j0 = 0; j0 < nrhs; j0 += kResidualBlock) {
-            const int kc = std::min(kResidualBlock, nrhs - j0);
-            const bool abs_here = with_anorm && j0 == 0;
-            CKI(launch_residual_block(dA, lda, n, dX + (long long)j0 * ldx, ldx, dB + (long long)j0 * ldb, ldb,
-                                      c->rb_R + (long long)j0 * n, n, kc, c->rb_partial, norms + 2 * j0, st,
-                                      abs_here ? c->rowsum_part : nullptr, abs_here ? c->anorm : nullptr));
-            c->kernel_launches += 2;
-        }
-        c->anorm_pending = false;
-        CK(cudaMemcpyAsync(h_norms.data(), norms, 3 * (size_t)nrhs * sizeof(double), cudaMemcpyDeviceToHost, st));
-        if (first_pass || with_anorm) CK(cudaMemcpyAsync(&anorm, c->anorm, sizeof(double), cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        bool all = true, nan = false;
-        for (int j = 0; j < nrhs; ++j) {
-            const double rn = h_norms[2 * j], xn = h_norms[2 * j + 1], bn = h_norms[2 * nrhs + j];
-            be[j] = backward_error(rn, anorm, xn, bn);
-            if (first_pass) first_be[j] = be[j];
-            const double thresh = c->opts.tol > 0 ? c->opts.tol * anorm * xn : xn * anorm * eps * std::sqrt((double)n);
-            if (!(rn == rn)) nan = true;
-            if (!(rn <= thresh)) all = false;
-        }
-        first_pass = false;
-        if (nan) break;  // NaN: give up
-        if (all) { converged = 1; break; }
-        if (iters >= max_iters) break;
-        if (c->opts.refinement == MPLU_REFINE_GMRES) {
-            for (int j = 0; j < nrhs; ++j) {
-                int inner = 0;
-                CKI(gmres_correction(c, dA, lda, c->rb_R + (long long)j * n, dX + (long long)j * ldx, &inner));
-                gmres_iters += inner;
-            }
-        } else {
-            CKI(solve_blocks(c->rb_R, n, nullptr, dX));
-        }
-        ++iters;
-    }
-    int h_status = 0;
-    CK(cudaMemcpy(&h_status, c->status, sizeof(int), cudaMemcpyDeviceToHost));
-    if (berr) std::copy(be.begin(), be.end(), berr);
-    if (stats) {
-        int w = 0;  // the worst column (a NaN is worse than anything)
-        for (int j = 1; j < nrhs; ++j)
-            if (be[j] > be[w] || (be[j] != be[j] && be[w] == be[w])) w = j;
-        stats->n = n;
-        stats->iters = iters;
-        stats->converged = converged;
-        stats->status_bits = h_status;
-        stats->anorm_inf = anorm;
-        stats->bnorm_inf = h_norms[2 * nrhs + w];
-        stats->xnorm_inf = h_norms[2 * w + 1];
-        stats->rnorm_inf = h_norms[2 * w];
-        stats->backward_error = be[w];
-        stats->first_backward_error = *std::max_element(first_be.begin(), first_be.end());
-        stats->gemm_launches = c->gemm_launches;
-        stats->kernel_launches = c->kernel_launches;
-        stats->trailing_launches = c->trail_count;
-        stats->trailing_flops = c->trail_flops;
-        stats->trailing_bytes = c->trail_bytes;
-        stats->gmres_iters = gmres_iters;
-        float tms = 0.f;
-        for (int i = 0; i < c->trail_count; ++i) {
-            float ms = 0.f;
-            if (cudaEventElapsedTime(&ms, c->trail_ev[2 * i], c->trail_ev[2 * i + 1]) == cudaSuccess) tms += ms;
-        }
-        stats->trailing_ms = tms;
-    }
-    if (converged) return 0;
-    if (h_status & 1) return MPLU_E_OVERFLOW;
-    if (h_status & 2) return MPLU_E_ZEROPIVOT;
-    return MPLU_E_NOCONV;
+int dsgesv_iter(int rc, int iters) {
+    return rc == 0 ? iters : (rc == MPLU_E_OVERFLOW ? -2 : (rc == MPLU_E_NOCONV ? -(iters + 1) : -3));
 }
 
 // The right-hand sides of one call: nrhs column-major columns of B (ldb) and X (ldx); berr: host array of nrhs or null.
-// nrhs = 1 goes through solve_impl, the single-vector path, unchanged.
 struct RhsBlock {
     int nrhs;
     const double* B; long long ldb;
@@ -1831,9 +1705,93 @@ struct RhsBlock {
     double* berr;
 };
 
-int solve_rhs(mplu_context* c, const double* dA, long long lda, const RhsBlock& b, mplu_stats* stats) {
-    if (b.nrhs == 1) return solve_impl(c, dA, lda, b.B, b.X, stats);
-    return solve_nrhs_impl(c, dA, lda, b.nrhs, b.B, b.ldb, b.X, b.ldx, b.berr, stats);
+// X = (LU)^-1 B, refined.  One column runs the single-vector kernels on c->r / c->norms.  More columns run the block
+// kernels on the rb_* buffers, which stream A and the factors once per kResidualBlock / kSolveBlock columns; GMRES
+// refinement runs gmres_correction column by column (not batched).
+int solve_impl(mplu_context* c, const double* dA, long long lda, const RhsBlock& b, mplu_stats* stats) {
+    if (!c->factored) return MPLU_E_NOTFACTORED;
+    const int n = c->n, npad = c->npad, k = b.nrhs;
+    const long long ld = npad;
+    cudaStream_t st = c->stream;
+    if (k > 1) CKI(ensure_rhs_work(c, k));
+    double* R = k == 1 ? c->r : c->rb_R;  // the residual columns (ld n)
+    double* norms = k == 1 ? c->norms : c->rb_norms;
+    // D = (LU)^-1 rhs: D -> d_out, or x_accum += D (both with ld b.ldx)
+    auto solve = [&](const double* rhs, long long ldr, double* d_out, double* x_accum) -> int {
+        if (k == 1) {
+            c->kernel_launches += 1;
+            return launch_lu_solve(c->W, ld, n, npad, c->Linv32, c->Uinv32, rhs, c->y, d_out, x_accum, c->ready, st);
+        }
+        for (int j0 = 0; j0 < k; j0 += kSolveBlock) {
+            const int kc = std::min(kSolveBlock, k - j0);
+            CKI(launch_lu_solve_block(c->W, ld, n, npad, c->Linv32, c->Uinv32, rhs + (long long)j0 * ldr, ldr, kc, c->rb_y,
+                                      d_out ? d_out + (long long)j0 * b.ldx : nullptr, b.ldx,
+                                      x_accum ? x_accum + (long long)j0 * b.ldx : nullptr, b.ldx, c->ready, st));
+            c->kernel_launches += 2;
+        }
+        return 0;
+    };
+    RefineOps ops;
+    ops.norms = norms;
+    ops.anorm = c->anorm;
+    ops.st = st;
+    ops.first_solve = [&]() -> int {
+        CKI(launch_column_absmax(b.B, b.ldb, n, k, norms + 2 * k, st));
+        c->kernel_launches += 1;
+        return solve(b.B, b.ldb, b.X, nullptr);
+    };
+    ops.residual = [&](bool* formed_anorm) -> int {
+        // lazy first touch: ||A||_inf rides in the first residual pass (of the first column block): it streams A anyway
+        const bool with_anorm = c->anorm_pending;
+        if (k == 1) {
+            CKI(launch_residual(dA, lda, n, b.X, b.B, R, c->partial, c->nchunk, norms, st, with_anorm ? c->rowsum_part : nullptr,
+                                with_anorm ? c->anorm : nullptr));
+            c->kernel_launches += 2;
+        } else {
+            for (int j0 = 0; j0 < k; j0 += kResidualBlock) {
+                const int kc = std::min(kResidualBlock, k - j0);
+                const bool abs_here = with_anorm && j0 == 0;
+                CKI(launch_residual_block(dA, lda, n, b.X + (long long)j0 * b.ldx, b.ldx, b.B + (long long)j0 * b.ldb, b.ldb,
+                                          R + (long long)j0 * n, n, kc, c->rb_partial, norms + 2 * j0, st,
+                                          abs_here ? c->rowsum_part : nullptr, abs_here ? c->anorm : nullptr));
+                c->kernel_launches += 2;
+            }
+        }
+        c->anorm_pending = false;
+        *formed_anorm = with_anorm;
+        return 0;
+    };
+    ops.correct = [&](int* krylov_steps) -> int {
+        if (c->opts.refinement != MPLU_REFINE_GMRES) return solve(R, n, nullptr, b.X);
+        for (int j = 0; j < k; ++j) {
+            int inner = 0;
+            CKI(gmres_correction(c, dA, lda, R + (long long)j * n, b.X + (long long)j * b.ldx, &inner));
+            *krylov_steps += inner;
+        }
+        return 0;
+    };
+    ops.wait = [&]() -> int { return (int)cudaStreamSynchronize(st); };
+    RefineResult res;
+    CKI(refine(ops, n, k, c->opts.max_iters, c->opts.tol, &res));
+    int h_status = 0;
+    CK(cudaMemcpy(&h_status, c->status, sizeof(int), cudaMemcpyDeviceToHost));
+    refine_stats(res, n, b.berr, stats);
+    if (stats) {
+        stats->status_bits = h_status;
+        stats->gmres_iters = res.gmres_iters;
+        stats->gemm_launches = c->gemm_launches;
+        stats->kernel_launches = c->kernel_launches;
+        stats->trailing_launches = c->trail_count;
+        stats->trailing_flops = c->trail_flops;
+        stats->trailing_bytes = c->trail_bytes;
+        float tms = 0.f;
+        for (int i = 0; i < c->trail_count; ++i) {
+            float ms = 0.f;
+            if (cudaEventElapsedTime(&ms, c->trail_ev[2 * i], c->trail_ev[2 * i + 1]) == cudaSuccess) tms += ms;
+        }
+        stats->trailing_ms = tms;
+    }
+    return refine_rc(res.converged, h_status);
 }
 
 // factor + solve from device-resident inputs with the cascade of LAPACK dsgesv: early-scale redo, bf16 on fp16 overflow,
@@ -1850,7 +1808,7 @@ int gesv_device_impl(mplu_context* c, int n, const double* dA, long long lda, co
     int rc = factor_impl(c, n, dA, lda);
     if (rc) return rc;
     CK(cudaEventRecord(c->ev[1], c->stream));
-    rc = solve_rhs(c, dA, lda, b, stats);
+    rc = solve_impl(c, dA, lda, b, stats);
     if (rc == MPLU_E_OVERFLOW && c->used_early_scale) {
         // the fp16 scale taken from the first block column did not fit a later one: once more with the global scale
         c->allow_early = false;
@@ -1859,7 +1817,7 @@ int gesv_device_impl(mplu_context* c, int n, const double* dA, long long lda, co
         c->allow_early = true;
         if (rc) return rc;
         if (stats) memset(stats, 0, sizeof(*stats));
-        rc = solve_rhs(c, dA, lda, b, stats);
+        rc = solve_impl(c, dA, lda, b, stats);
     }
     if (rc == MPLU_E_OVERFLOW && c->opts.precision == MPLU_FP16 && c->opts.bf16_fallback) {
         // like dsgesv's fall back to full precision: same algorithm, operand type without the range problem
@@ -1868,11 +1826,11 @@ int gesv_device_impl(mplu_context* c, int n, const double* dA, long long lda, co
         rc = factor_impl(c, n, dA, lda);
         if (rc) return rc;
         if (stats) memset(stats, 0, sizeof(*stats));
-        rc = solve_rhs(c, dA, lda, b, stats);
+        rc = solve_impl(c, dA, lda, b, stats);
     }
     if (stats) {
         stats->precision_used = c->opts.precision;
-        stats->dsgesv_iter = rc == 0 ? stats->iters : (rc == MPLU_E_OVERFLOW ? -2 : (rc == MPLU_E_NOCONV ? -(stats->iters + 1) : -3));
+        stats->dsgesv_iter = dsgesv_iter(rc, stats->iters);
     }
     if ((rc == MPLU_E_OVERFLOW || rc == MPLU_E_ZEROPIVOT || rc == MPLU_E_NOCONV) && c->opts.fp64_fallback)
         rc = fp64_fallback_solve(c, n, dA, lda, b.nrhs, b.B, b.ldb, b.X, b.ldx, rc, b.berr, stats);  // dsgesv: full-precision factorization and solve
@@ -1931,10 +1889,10 @@ int gesv_host_impl(mplu_context* c, int n, const double* hA, long long lda, cons
         rc = factor_streamed(c, n, hA, lda, c->dA_stage);
         if (rc) return rc;
         CK(cudaEventRecord(c->ev[1], st));
-        rc = solve_rhs(c, c->dA_stage, n, db, stats);
+        rc = solve_impl(c, c->dA_stage, n, db, stats);
         if (stats) {
             stats->precision_used = c->opts.precision;
-            stats->dsgesv_iter = rc == 0 ? stats->iters : (rc == MPLU_E_OVERFLOW ? -2 : (rc == MPLU_E_NOCONV ? -(stats->iters + 1) : -3));
+            stats->dsgesv_iter = dsgesv_iter(rc, stats->iters);
         }
         if ((rc == MPLU_E_ZEROPIVOT || rc == MPLU_E_NOCONV) && c->opts.fp64_fallback)
             rc = fp64_fallback_solve(c, n, c->dA_stage, n, db.nrhs, db.B, db.ldb, db.X, db.ldx, rc, db.berr, stats);
@@ -1981,11 +1939,6 @@ bool columns_overlap(const double* B, long long ldb, const double* X, long long 
     const double* b1 = B + (long long)(nrhs - 1) * ldb + n;
     const double* x1 = X + (long long)(nrhs - 1) * ldx + n;
     return X < b1 && B < x1;
-}
-
-// berr of a one-column call, from the single-vector path's stats
-void single_berr(const mplu_stats* stats, double* berr) {
-    if (berr) berr[0] = backward_error(stats->rnorm_inf, stats->anorm_inf, stats->xnorm_inf, stats->bnorm_inf);
 }
 
 }  // namespace mplu_detail
@@ -2060,8 +2013,8 @@ int mplu_create(mplu_context** out, int device) {
         for (auto& e : c->ev) CK(cudaEventCreate(&e));
         CK(cudaMalloc(&c->scales, SC_COUNT * sizeof(float)));
         CK(cudaMalloc(&c->amax, sizeof(float)));
-        CK(cudaMalloc(&c->anorm, 2 * sizeof(double)));
-        CK(cudaMalloc(&c->norms, 2 * sizeof(double)));
+        CK(cudaMalloc(&c->anorm, sizeof(double)));
+        CK(cudaMalloc(&c->norms, 3 * sizeof(double)));
         CK(cudaMalloc(&c->status, sizeof(int)));
         CK(cudaMalloc(&c->ready, sizeof(unsigned)));
         return 0;
@@ -2116,7 +2069,7 @@ int mplu_solve_device(mplu_context* c, const double* dA, long long lda, const do
     if (!c || !dA || !db || !dx) return MPLU_E_ARG;
     CK(cudaSetDevice(c->device));
     if (stats) memset(stats, 0, sizeof(*stats));
-    return solve_impl(c, dA, lda, db, dx, stats);
+    return solve_impl(c, dA, lda, RhsBlock{1, db, c->n, dx, c->n, nullptr}, stats);
 }
 
 int mplu_gesv_device(mplu_context* c, int n, const double* dA, long long lda, const double* db, double* dx,
@@ -2136,34 +2089,22 @@ int mplu_solve_device_nrhs(mplu_context* c, int nrhs, const double* dA, long lon
     if (!c || !dA || !dB || !dX || nrhs < 1 || lda < c->n || ldb < c->n || ldx < c->n) return MPLU_E_ARG;
     if (columns_overlap(dB, ldb, dX, ldx, c->n, nrhs)) return MPLU_E_ARG;
     CK(cudaSetDevice(c->device));
-    mplu_stats local;
-    if (!stats) stats = &local;
-    memset(stats, 0, sizeof(*stats));
-    const int rc = solve_rhs(c, dA, lda, RhsBlock{nrhs, dB, ldb, dX, ldx, berr}, stats);
-    if (nrhs == 1) single_berr(stats, berr);
-    return rc;
+    if (stats) memset(stats, 0, sizeof(*stats));
+    return solve_impl(c, dA, lda, RhsBlock{nrhs, dB, ldb, dX, ldx, berr}, stats);
 }
 
 int mplu_gesv_device_nrhs(mplu_context* c, int n, int nrhs, const double* dA, long long lda, const double* dB, long long ldb,
                           double* dX, long long ldx, const mplu_options* opts, double* berr, mplu_stats* stats) {
     if (!c || !dA || !dB || !dX || n <= 0 || nrhs < 1 || lda < n || ldb < n || ldx < n) return MPLU_E_ARG;
     if (columns_overlap(dB, ldb, dX, ldx, n, nrhs)) return MPLU_E_ARG;
-    mplu_stats local;
-    if (!stats) stats = &local;
-    const int rc = gesv_device_impl(c, n, dA, lda, RhsBlock{nrhs, dB, ldb, dX, ldx, berr}, opts, stats);
-    if (nrhs == 1) single_berr(stats, berr);
-    return rc;
+    return gesv_device_impl(c, n, dA, lda, RhsBlock{nrhs, dB, ldb, dX, ldx, berr}, opts, stats);
 }
 
 int mplu_gesv_host_nrhs(mplu_context* c, int n, int nrhs, const double* hA, long long lda, const double* hB, long long ldb,
                         double* hX, long long ldx, const mplu_options* opts, double* berr, mplu_stats* stats) {
     if (!c || !hA || !hB || !hX || n <= 0 || nrhs < 1 || lda < n || ldb < n || ldx < n) return MPLU_E_ARG;
     if (columns_overlap(hB, ldb, hX, ldx, n, nrhs)) return MPLU_E_ARG;
-    mplu_stats local;
-    if (!stats) stats = &local;
-    const int rc = gesv_host_impl(c, n, hA, lda, RhsBlock{nrhs, hB, ldb, hX, ldx, berr}, opts, stats);
-    if (nrhs == 1) single_berr(stats, berr);
-    return rc;
+    return gesv_host_impl(c, n, hA, lda, RhsBlock{nrhs, hB, ldb, hX, ldx, berr}, opts, stats);
 }
 
 int mplu_get_factors(mplu_context* c, double* LU, long long ldlu, int on_device) {

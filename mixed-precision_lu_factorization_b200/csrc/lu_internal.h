@@ -6,6 +6,7 @@
 #include "getrf_fused.h"
 #include "kernels.h"
 
+#include <functional>
 #include <vector>
 
 // dry-run trace of a schedule (lu.cu: trace_*; tests/test_schedule_trace.py)
@@ -36,14 +37,14 @@ struct mplu_context {
     float* inv_scales = nullptr;  // 4 per diagonal block
     float* scales = nullptr;      // SC_COUNT
     float* amax = nullptr;
-    double* anorm = nullptr;      // [0] ||A||inf, [1] ||b||inf
+    double* anorm = nullptr;      // ||A||inf
     double* rowsum_part = nullptr;
     int* status = nullptr;
     unsigned* ready = nullptr;    // step counter of the cooperative triangular-solve kernel
     // refinement
     double* r = nullptr;
     double* partial = nullptr;
-    double* norms = nullptr;  // [0] ||r||, [1] ||x||
+    double* norms = nullptr;  // [0] ||r||, [1] ||x||, [2] ||b|| (the layout of RefineOps::norms for one column)
     float* y = nullptr;       // 2*npad
     int nchunk = 64;
     // several right-hand sides (mplu_*_nrhs): allocated on the first call with nrhs > 1, freed with the other work arrays
@@ -197,5 +198,34 @@ int fp64_fallback_solve(mplu_context* c, int n, const double* dA, long long lda,
                         double* dX, long long ldx, int why, double* berr, mplu_stats* stats);
 // the per-column backward error ||r|| / (||A|| ||x|| + ||b||) (0 for r = 0: a zero column is solved exactly)
 inline double backward_error(double rn, double an, double xn, double bn) { return rn == 0.0 ? 0.0 : rn / (an * xn + bn); }
+
+// LAPACK dsgesv's iterative refinement of k columns that share the iteration count (refine, lu.cu).  The caller enqueues
+// the device work; refine reads the norms back, applies the stopping rule and counts.  Every operation returns 0 or an
+// error code.
+struct RefineOps {
+    // device norms, read back on st: [2j] ||r_j||_inf, [2j+1] ||x_j||_inf, [2k+j] ||b_j||_inf; and ||A||_inf
+    const double* norms;
+    const double* anorm;
+    cudaStream_t st;
+    std::function<int()> first_solve;                 // the ||b_j|| and X = (LU)^-1 B
+    std::function<int(bool* formed_anorm)> residual;  // R = B - A X and its norms; *formed_anorm: this pass also formed ||A||
+    std::function<int(int* krylov_steps)> correct;    // X += the correction computed from R
+    std::function<int()> wait;                        // until the norms have arrived on the host
+};
+struct RefineColumn { double rnorm, xnorm, bnorm, berr, first_berr; };
+struct RefineResult {
+    std::vector<RefineColumn> col;
+    double anorm = 0.0;
+    int iters = 0, converged = 0, gmres_iters = 0;
+};
+// max_iters <= 0: dsgesv's 30.  tol <= 0: ||r_j|| <= ||x_j|| ||A|| eps sqrt(n), else ||r_j|| <= tol ||A|| ||x_j||
+int refine(const RefineOps& ops, int n, int k, int max_iters, double tol, RefineResult* res);
+// berr (host, may be null) = every column's backward error; the refinement fields of stats (may be null) = those of the
+// worst column (the largest backward error, the first NaN), first_backward_error = the largest first-solve one
+void refine_stats(const RefineResult& res, int n, double* berr, mplu_stats* stats);
+// 0 when converged, else what the status bits of the factorization explain, else MPLU_E_NOCONV
+int refine_rc(int converged, int status_bits);
+// LAPACK dsgesv's ITER for a mixed-precision solve that ended with rc after iters corrections
+int dsgesv_iter(int rc, int iters);
 
 }  // namespace mplu_detail

@@ -80,6 +80,10 @@ def test_block_cyclic_bf16_and_no_lookahead(mplu, single_ref):
             xs, st = ds.gesv(n, nb, As, bs, mplu.default_options(**kw))
             assert st.converged == 1 and st.backward_error <= 2 * n * EPS
             np.testing.assert_allclose(xs[0].cpu().numpy(), single_ref[n]["x_ref"], rtol=0, atol=1e-12)
+        # b = 0: x = 0 solves it exactly, so the backward error is 0, as in the single-GPU path
+        xs, st = ds.gesv(n, nb, As, [b.new_zeros(n) for b in bs], mplu.default_options())
+        assert st.converged == 1 and st.backward_error == 0.0 and st.first_backward_error == 0.0
+        assert all((x == 0).all() for x in xs)
     finally:
         ds.close()
 

@@ -26,12 +26,12 @@ def system(oracle, n, nrhs, seed=0):
     return A, Xt, A @ Xt
 
 
-def gesv_nrhs(mplu, solver, A, B, **kw):
+def gesv_nrhs(mplu, solver, A, B, allow_noconv=False, **kw):
     import torch
     dA, dB = dev(A), dev(B)
     B0 = dB.clone()
-    X, st, berr = solver.gesv_nrhs(dA, dB, mplu.default_options(**kw))
-    assert torch.equal(dB, B0)  # B is not modified
+    X, st, berr = solver.gesv_nrhs(dA, dB, mplu.default_options(**kw), allow_noconv)
+    assert torch.equal(dB.view(torch.int64), B0.view(torch.int64))  # B is not modified (bit for bit: B may hold a NaN)
     return X.cpu().numpy(), st, berr
 
 
@@ -67,6 +67,20 @@ def test_one_column_is_the_single_vector_path(mplu, oracle, solver):
     assert torch.equal(x3, X4)
     skip = TIMING | {"kernel_launches"}  # the launch counter runs on across solves with the same factors
     assert {k: v for k, v in s3.as_dict().items() if k not in skip} == {k: v for k, v in s4.as_dict().items() if k not in skip}
+    # b = 0: x = 0 solves it exactly, so the backward error is 0, as for a zero column of a block
+    z = torch.zeros(n, dtype=torch.float64, device="cuda")
+    x5, s5 = solver.gesv(dA, z, mplu.default_options())
+    X6, s6, berr6 = solver.gesv_nrhs(dA, cm(z.reshape(n, 1)), mplu.default_options())
+    torch.cuda.synchronize()
+    s7 = solver.solve_ptr(dA.data_ptr(), n, z.data_ptr(), x3.data_ptr())
+    for s in (s5, s6, s7):
+        assert s.converged == 1 and s.backward_error == 0.0 and s.first_backward_error == 0.0
+    assert (x5 == 0).all() and (X6 == 0).all() and (x3 == 0).all() and berr6[0] == 0.0
+    # ||b||_inf keeps a NaN of b, like the column norms of a block
+    z[n // 2] = float("nan")
+    torch.cuda.synchronize()
+    s8 = solver.solve_ptr(dA.data_ptr(), n, z.data_ptr(), x3.data_ptr(), allow_noconv=True)
+    assert np.isnan(s8.bnorm_inf)
 
 
 def test_column_independence(mplu, oracle, solver):
@@ -148,13 +162,13 @@ def test_full_precision_fallback(mplu, oracle, solver, host):
     n, nrhs = 512, 4
     rng = np.random.default_rng(3)
 
-    def solve(A, B, **kw):
+    def solve(A, B, allow_noconv=False, **kw):
         if host:
             hA, hB, hX = np.asfortranarray(A), np.asfortranarray(B), np.empty((n, nrhs), order="F")
             st, berr = solver.gesv_host_nrhs_ptr(n, nrhs, hA.ctypes.data, n, hB.ctypes.data, n, hX.ctypes.data, n,
-                                                 mplu.default_options(**kw))
+                                                 mplu.default_options(**kw), allow_noconv)
             return hX, st, berr
-        return gesv_nrhs(mplu, solver, A, B, **kw)
+        return gesv_nrhs(mplu, solver, A, B, allow_noconv, **kw)
 
     A = rng.standard_normal((n, n)) + 30.0 * np.eye(n)
     A[0, 0] = 0.0
@@ -172,6 +186,14 @@ def test_full_precision_fallback(mplu, oracle, solver, host):
     X3, st3, berr3 = solve(A3, A3 @ Xt)
     assert st3.fp64_fallback == 0 and st3.dsgesv_iter == st3.iters >= 1 and st3.converged == 1
     assert (berr3 <= 2 * n * EPS).all()
+    # two columns end in NaN (an Inf and a NaN in b): the stats describe the first of them
+    B4 = A @ Xt
+    B4[5, 1] = np.inf
+    B4[9, 2] = np.nan
+    X4, st4, berr4 = solve(A, B4, allow_noconv=True)
+    assert st4.fp64_fallback == 1 and st4.dsgesv_iter == -3 and st4.converged == 0
+    assert np.isnan(berr4[1]) and np.isnan(berr4[2]) and (berr4[[0, 3]] <= 2 * n * EPS).all()
+    assert np.isnan(st4.backward_error) and st4.bnorm_inf == np.inf
 
 
 def test_fp16_overflow_falls_back_to_bf16(mplu, oracle, solver):

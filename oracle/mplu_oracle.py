@@ -362,6 +362,108 @@ def lu_solve(LU: np.ndarray, b: np.ndarray, dtype=np.float32) -> np.ndarray:
     return solve_triangular(LU, y, lower=False, check_finite=False)
 
 
+def factor_tile_ratio(A, LU, tile: int = 128):
+    """Componentwise backward error of a no-pivot factorization, tile by tile: with L = tril(LU,-1) + I, U = triu(LU),
+    E = |L U - A| and M = |L| |U| (fp64), returns rho[I, J] = max E_IJ / max M_IJ over the tile x tile tiles (the last
+    row / column of tiles is ragged when n is not a multiple of `tile`).  A tile whose M is all zero must have E = 0:
+    its rho is 0 then, inf otherwise.  Unlike a bound relative to max|LU| (the diagonal, on dominant inputs) it does not
+    let a wrong off-diagonal tile hide behind a large diagonal.  numpy arrays or torch tensors; CUDA tensors stay on the
+    device and the result is a numpy array either way."""
+    try:
+        import torch
+    except ImportError:
+        torch = None
+    if torch is not None and (isinstance(A, torch.Tensor) or isinstance(LU, torch.Tensor)):
+        dev = LU.device if isinstance(LU, torch.Tensor) else A.device
+        A = torch.as_tensor(A, dtype=torch.float64, device=dev)
+        LU = torch.as_tensor(LU, dtype=torch.float64, device=dev)
+        n = LU.shape[0]
+        L = torch.tril(LU, -1) + torch.eye(n, dtype=torch.float64, device=dev)
+        U = torch.triu(LU)
+        E = (L @ U - A).abs()
+        M = L.abs() @ U.abs()
+        del L, U
+        npad = -(-n // tile) * tile
+        E = torch.nn.functional.pad(E, (0, npad - n, 0, npad - n))
+        M = torch.nn.functional.pad(M, (0, npad - n, 0, npad - n))
+        nt = npad // tile
+        Emax = E.reshape(nt, tile, nt, tile).amax(dim=(1, 3)).cpu().numpy()
+        Mmax = M.reshape(nt, tile, nt, tile).amax(dim=(1, 3)).cpu().numpy()
+    else:
+        A = np.asarray(A, dtype=np.float64)
+        LU = np.asarray(LU, dtype=np.float64)
+        n = LU.shape[0]
+        L = np.tril(LU, -1) + np.eye(n)
+        U = np.triu(LU)
+        npad = -(-n // tile) * tile
+        E = np.zeros((npad, npad))
+        M = np.zeros((npad, npad))
+        E[:n, :n] = np.abs(L @ U - A)
+        M[:n, :n] = np.abs(L) @ np.abs(U)
+        nt = npad // tile
+        Emax = E.reshape(nt, tile, nt, tile).max(axis=(1, 3))
+        Mmax = M.reshape(nt, tile, nt, tile).max(axis=(1, 3))
+    with np.errstate(divide="ignore", invalid="ignore"):
+        return np.where(Mmax > 0, Emax / np.where(Mmax > 0, Mmax, 1.0), np.where(Emax == 0, 0.0, np.inf))
+
+
+def factor_tile_distance(LU, LU_ref, tile: int = 128):
+    """How far two factorizations of the same matrix are apart, in the units of factor_tile_ratio: per tile
+    max|L U - L_ref U_ref| / max(|L| |U|).  Two schedules documented to form the same products up to fp32 rounding
+    must stay far below the factors' own backward error here; a wrong tile in one of them shows at its own size even
+    where it stays under the backward-error bound.  numpy arrays or torch tensors (CUDA tensors stay on the device)."""
+    try:
+        import torch
+    except ImportError:
+        torch = None
+    if torch is not None and isinstance(LU_ref, torch.Tensor):
+        n = LU_ref.shape[0]
+        R = LU_ref.to(torch.float64)
+        P = (torch.tril(R, -1) + torch.eye(n, dtype=torch.float64, device=R.device)) @ torch.triu(R)
+    else:
+        R = np.asarray(LU_ref, dtype=np.float64)
+        P = (np.tril(R, -1) + np.eye(R.shape[0])) @ np.triu(R)
+    return factor_tile_ratio(P, LU, tile)
+
+
+def blocked_sweeps(LU, Linv, Uinv, B, dtype=np.float64, store=np.float32, blk: int = 128):
+    """Host restatement of the device triangular solve L U X = B (lu_solve_kernel, lu_solve_block_kernel in csrc/ir.cu).
+    LU: n x n factors (the fp32 working matrix, widened); Linv / Uinv: the device's fp32 inverses of the unit-lower /
+    upper diagonal blk-blocks, shape (npad/blk, blk, blk); B: n or n x k.  The order is padded to npad = ceil(n/blk)*blk
+    with identity factors and a zero right-hand side, the right-hand side is cast to fp32 (static_cast<float>(rhs[row]))
+    and the two sweeps are left-looking over block rows:
+        forward   y_i = Linv_i (b_i - sum_{j<i} L_ij y_j)
+        backward  x_i = Uinv_i (y_i - sum_{j>i} U_ij x_j)
+    Each solved block is rounded to `store` (the kernels keep ysol / xsol in fp32); everything else is evaluated in `dtype`:
+    fp64 gives the reference, fp32 a same-order evaluation whose distance from it sizes the kernels' own rounding.
+    Returns X in fp64 with B's shape."""
+    LU = np.asarray(LU, dtype=np.float64)
+    B = np.asarray(B, dtype=np.float64)
+    vec = B.ndim == 1
+    B = B.reshape(B.shape[0], -1)
+    n, k = B.shape
+    npad = -(-n // blk) * blk
+    nblk = npad // blk
+    F = np.eye(npad, dtype=dtype)
+    F[:n, :n] = LU
+    Li = np.asarray(Linv, dtype=dtype).reshape(nblk, blk, blk)
+    Ui = np.asarray(Uinv, dtype=dtype).reshape(nblk, blk, blk)
+    rhs = np.zeros((npad, k), dtype=dtype)
+    rhs[:n] = B.astype(np.float32)
+    y = np.zeros((npad, k), dtype=dtype)
+    x = np.zeros((npad, k), dtype=dtype)
+    for i in range(nblk):
+        r = slice(i * blk, (i + 1) * blk)
+        acc = rhs[r] - F[r, :i * blk] @ y[:i * blk]
+        y[r] = (Li[i] @ acc).astype(store)
+    for i in reversed(range(nblk)):
+        r = slice(i * blk, (i + 1) * blk)
+        acc = y[r] - F[r, (i + 1) * blk:] @ x[(i + 1) * blk:]
+        x[r] = (Ui[i] @ acc).astype(store)
+    X = x[:n].astype(np.float64)
+    return X[:, 0] if vec else X
+
+
 def refine(A: np.ndarray, b: np.ndarray, LU: np.ndarray, max_iters: int = 30, tol: float = 0.0):
     """fp64 iterative refinement with low-precision factors and LAPACK dsgesv's stopping rule
     ||r||_inf <= ||x||_inf ||A||_inf eps sqrt(n).  Returns dict(x, iters, converged, backward_error, first)."""

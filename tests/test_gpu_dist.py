@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT
+from test_gpu_reference import check_factors
 
 pytestmark = pytest.mark.gpu
 EPS = np.finfo(np.float64).eps / 2
@@ -35,7 +36,7 @@ def single_ref(mplu, oracle):
 
 @pytest.mark.parametrize("n,nb,P,Q", [(1024, 256, 1, 1), (1024, 256, 1, 2), (1024, 256, 2, 2), (1024, 256, 2, 4),
                                       (2048, 256, 2, 2), (2048, 512, 2, 4), (1024, 128, 3, 2)])
-def test_block_cyclic_solve_matches_single_gpu_and_lapack(mplu, oracle, single_ref, n, nb, P, Q):
+def test_block_cyclic_solve_matches_single_gpu_and_lapack(mplu, oracle, single_ref, record_property, n, nb, P, Q):
     ref = single_ref[n]
     ds = mplu.DistSolver(0, P, Q)
     try:
@@ -67,6 +68,7 @@ def test_block_cyclic_solve_matches_single_gpu_and_lapack(mplu, oracle, single_r
         assert np.abs(np.triu(LU) - np.triu(lu_ref)).max() <= 0.02 * u16 * np.abs(lu_ref).max()
         assert np.abs(np.tril(LU, -1) - np.tril(lu_ref, -1)).max() <= 2 * u16 * np.abs(np.tril(lu_ref, -1)).max()
         assert np.abs(np.triu(LU) - np.triu(ref["LU"])).max() <= 0.02 * u16 * np.abs(lu_ref).max()
+        check_factors(oracle, record_property, ref["A"], LU, 0)  # tile by tile: blind to no off-diagonal tile
     finally:
         ds.close()
 

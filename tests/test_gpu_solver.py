@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN
+from test_gpu_reference import check_agreement, check_factors
 
 pytestmark = pytest.mark.gpu
 
@@ -26,7 +27,7 @@ def run(mplu, solver, A, b, **kw):
 
 @pytest.mark.parametrize("n", [1024])
 @pytest.mark.parametrize("precision", [0, 1])
-def test_config1_n1024_vs_lapack_and_oracle(mplu, oracle, solver, n, precision):
+def test_config1_n1024_vs_lapack_and_oracle(mplu, oracle, solver, record_property, n, precision):
     """BASELINE.json configs[0]: n=1024 diagonally dominant, no-pivot LU + IR single RHS vs host dgetrf/dgetrs."""
     A = oracle.counter_matrix(n, seed=1)
     b = A.sum(axis=1)
@@ -45,6 +46,7 @@ def test_config1_n1024_vs_lapack_and_oracle(mplu, oracle, solver, n, precision):
     u16 = 2.0 ** -11 if precision == 0 else 2.0 ** -8
     assert np.abs(np.triu(LU) - np.triu(lu_ref)).max() <= 0.02 * u16 * np.abs(lu_ref).max()
     assert np.abs(np.tril(LU, -1) - np.tril(lu_ref, -1)).max() <= 2 * u16 * np.abs(np.tril(lu_ref, -1)).max()
+    check_factors(oracle, record_property, A, LU, precision)
 
 
 @pytest.mark.parametrize("n", [128, 256])
@@ -73,7 +75,7 @@ def test_ragged_sizes(mplu, oracle, solver, n):
 
 @pytest.mark.parametrize("nb", [128, 256, 1024, 2048])
 @pytest.mark.parametrize("variant", [0, 1])
-def test_block_sizes_and_gemm_variants_agree(mplu, oracle, solver, nb, variant):
+def test_block_sizes_and_gemm_variants_agree(mplu, oracle, solver, record_property, nb, variant):
     n = 2304
     A = oracle.counter_matrix(n, seed=4)
     b = A.sum(axis=1)
@@ -81,6 +83,7 @@ def test_block_sizes_and_gemm_variants_agree(mplu, oracle, solver, nb, variant):
     assert st["converged"] == 1 and st["iters"] <= 3
     assert st["backward_error"] <= 2 * n * EPS
     assert np.abs(x - 1).max() < 1e-11
+    check_factors(oracle, record_property, A, solver.factors(n), 0)
 
 
 def test_solve_reuses_factors_for_new_rhs(mplu, oracle, solver):
@@ -113,7 +116,7 @@ def test_host_buffer_entry_point(mplu, oracle, solver):
 
 @pytest.mark.parametrize("n,nb", [(2304, 512), (1000, 256), (4096, 1024)])
 @pytest.mark.parametrize("pinned", [False, True])
-def test_streamed_host_path_gives_bit_identical_factors(mplu, oracle, n, nb, pinned):
+def test_streamed_host_path_gives_bit_identical_factors(mplu, oracle, record_property, n, nb, pinned):
     """mplu_gesv_host factors left-looking, block column by block column, while A is still arriving over PCIe: the same
     products in the same order as the device schedule, hence the same factors bit for bit and the same solution;
     stream_host=0 (copy first, then the device schedule) is the comparison."""
@@ -142,11 +145,12 @@ def test_streamed_host_path_gives_bit_identical_factors(mplu, oracle, n, nb, pin
             assert it == outs[0][2]
             np.testing.assert_array_equal(xs, outs[0][1])
         np.testing.assert_allclose(outs[0][1], 1.0, rtol=0, atol=1e-11)
+        check_factors(oracle, record_property, A, outs[0][0], 0)
     finally:
         s.close()
 
 
-def test_streamed_host_path_scale_overflow_is_redone(mplu, oracle):
+def test_streamed_host_path_scale_overflow_is_redone(mplu, oracle, record_property):
     """The fp16 scale of the streamed path comes from the first block column; a later block column far outside that
     range must end in a correct solve (redo with the global scale), not in a silent overflow."""
     n, nb = 1536, 512
@@ -159,11 +163,13 @@ def test_streamed_host_path_scale_overflow_is_redone(mplu, oracle):
         st = s.gesv_host_ptr(n, A.ctypes.data, n, b.ctypes.data, x.ctypes.data, mplu.default_options(nb=nb))
         assert st.converged == 1
         np.testing.assert_allclose(x, 1.0, rtol=0, atol=1e-10)
+        if st.status_bits == 0:  # an overflow that did not spoil the solve keeps its factors on purpose
+            check_factors(oracle, record_property, A, s.factors(n), 0)
     finally:
         s.close()
 
 
-def test_early_scale_option(mplu, oracle, solver):
+def test_early_scale_option(mplu, oracle, solver, record_property):
     """early_scale=1 (left-looking schedule): the first touch overlaps the first diagonal tile, so the fp16 scale comes
     from the first block column.  Later block columns 2^6 larger leave the fp16 range under it: the overflow is
     reported (status bit 0) and, had it spoiled the solve, redone with the global scale; the answer must be right
@@ -173,8 +179,11 @@ def test_early_scale_option(mplu, oracle, solver):
     A[:, nb:] *= 64.0
     b = A.sum(axis=1)
     x1, st1 = run(mplu, solver, A, b, nb=nb, early_scale=1, lazy_touch=0)  # (the lazy first touch has its own test)
+    if st1["status_bits"] == 0:  # an overflow that did not spoil the solve keeps its factors on purpose
+        check_factors(oracle, record_property, A, solver.factors(n), 0, "rho_early")
     x0, st0 = run(mplu, solver, A, b, nb=nb, early_scale=0, lazy_touch=0)
     assert st0["converged"] == 1 and st0["status_bits"] == 0 and st0["precision_used"] == mplu.MPLU_FP16
+    check_factors(oracle, record_property, A, solver.factors(n), 0, "rho_global")
     assert st1["converged"] == 1
     np.testing.assert_allclose(x1, x0, rtol=0, atol=1e-11)
     np.testing.assert_allclose(x1, 1.0, rtol=0, atol=1e-10)
@@ -273,7 +282,7 @@ def test_full_size_properties_n32768(mplu, solver):
 
 
 @pytest.mark.parametrize("precision", [0, 1])
-def test_config2_n8192_factors_reproduce_A(mplu, solver, precision):
+def test_config2_n8192_factors_reproduce_A(mplu, oracle, solver, record_property, precision):
     """BASELINE.json configs[1] (n=8192, fp16 panel + fp16/fp32-accumulate GEMM + fp64 IR): L*U reproduces A to the
     16-bit operand tolerance, the refined solution to fp64."""
     import torch
@@ -287,8 +296,10 @@ def test_config2_n8192_factors_reproduce_A(mplu, solver, precision):
     U = torch.triu(LU)
     E = (L @ U - A).abs().max().item()
     u16 = 2.0 ** -11 if precision == 0 else 2.0 ** -8
-    # |A - LU| <= c * u16 * max|A| with a modest constant: the diagonal of this matrix is ~n/2 * 10
+    # |A - LU| <= c * u16 * max|A| with a modest constant: the diagonal of this matrix is ~n/2 * 10, kept to fp32 level
     assert E <= 0.05 * u16 * A.abs().max().item(), E
+    # and tile by tile against |L||U|: the bound above does not see a wrong off-diagonal tile (entries at most 9.9)
+    check_factors(oracle, record_property, A, LU, precision)
 
 
 # ---- condition-number sweep (BASELINE.json configs[4]) and GMRES-based refinement -----------------------------------
@@ -339,7 +350,7 @@ def test_fp16_overflow_falls_back_to_bf16(mplu, oracle, solver):
     assert np.isfinite(x2.cpu().numpy()).all()
 
 
-def test_schedule_options_do_not_change_the_arithmetic(mplu, oracle):
+def test_schedule_options_do_not_change_the_arithmetic(mplu, oracle, record_property):
     """Grouped launches, triangular K-range skipping, lane split, CUDA graph, workspace GETRF, the left-looking schedule
     (schedule=1), chain-lane programmatic launches and the width / grid of the persistent GETRF launches only change WHEN and
     WHERE the same products are formed: the factors are bit-identical within each GETRF arithmetic -- the dataflow launch
@@ -388,13 +399,15 @@ def test_schedule_options_do_not_change_the_arithmetic(mplu, oracle):
         for g in ("flow", "flow256"):  # another summation order on the same 16-bit operands
             d = (ref[g] - ref["unfused"]).abs().max().item()
             assert 0 <= d <= 2.0 ** -9 * m, (g, d)
+        for g, LU in ref.items():
+            check_factors(oracle, record_property, dA, LU, 0, f"rho_{g}")
     finally:
         s.close()
 
 
 @pytest.mark.parametrize("n,nb,fuse_w,ctas", [(4096, 2048, 2048, 16), (4096, 2048, 1024, 8), (4096, 4096, 4096, 16), (3000, 1024, 1024, 4)])
 @pytest.mark.parametrize("precision", [0, 1])
-def test_fused_getrf_matches_the_launch_per_product_path(mplu, oracle, n, nb, fuse_w, ctas, precision):
+def test_fused_getrf_matches_the_launch_per_product_path(mplu, oracle, record_property, n, nb, fuse_w, ctas, precision):
     """opts.fuse_w: the GETRF of a diagonal block (leaves + every product between them) as ONE persistent launch with grid
     barriers between the steps (csrc/getrf_fused.cu) instead of one launch per leaf / product group.  The products
     between the leaves are the same tcgen05 products on the same 16-bit operands in the same order; inside a leaf the
@@ -422,6 +435,8 @@ def test_fused_getrf_matches_the_launch_per_product_path(mplu, oracle, n, nb, fu
         assert dU <= 1e-5 * LU0.abs().max().item(), dU  # a few dozen fp32 ulps of the diagonal: the summation order differs
         # the 16-bit inverse of a diagonal block can round the other way: one fp16 ulp of a multiplier
         assert dL <= (2.0 ** -10 if precision == 0 else 2.0 ** -7) * torch.tril(LU0, -1).abs().max().item(), dL
+        check_factors(oracle, record_property, A, LU0, precision, "rho_unfused")
+        check_factors(oracle, record_property, A, LU1, precision, "rho_fused")
         assert float((x1 - 1).abs().max()) < 1e-11 and float((x1 - x0).abs().max()) < 1e-11
     finally:
         s.close()
@@ -429,7 +444,7 @@ def test_fused_getrf_matches_the_launch_per_product_path(mplu, oracle, n, nb, fu
 
 @pytest.mark.parametrize("n,nb", [(8192, 1024), (4096, 512), (6000, 1024), (16384, 2048)])
 @pytest.mark.parametrize("kw", [dict(), dict(lazy_touch=0), dict(use_graph=0, precision=1), dict(edge_nb=256, eager=0)])
-def test_paired_updates(mplu, oracle, n, nb, kw):
+def test_paired_updates(mplu, oracle, record_property, n, nb, kw):
     """opts.update_pair: two consecutive rank-nb updates of a block-column range applied as ONE product over both panels
     (K = 2 nb).  Same 16-bit products; the two partial sums meet in the TMEM accumulator instead of in fp32 C, so the factors
     agree with the one-update-per-pass schedule to fp32 rounding of the entries (not bit for bit), the refined solution to
@@ -453,13 +468,16 @@ def test_paired_updates(mplu, oracle, n, nb, kw):
         assert (LU1 - LU0).abs().max().item() <= tol * LU0.abs().max().item()
         assert float((x1 - 1).abs().max()) < 1e-11 and float((x1 - x0).abs().max()) < 1e-11
         assert st1.backward_error <= 2 * n * EPS
+        check_factors(oracle, record_property, A, LU0, kw.get("precision", 0), "rho_reference")
+        check_factors(oracle, record_property, A, LU1, kw.get("precision", 0))
+        check_agreement(oracle, record_property, LU1, LU0, kw.get("precision", 0))  # tile by tile, within AGREE
     finally:
         s.close()
 
 
 @pytest.mark.parametrize("n,nb,edge", [(8192, 1024, 512), (4096, 512, 128), (6000, 1024, 256), (16384, 2048, 1024)])
 @pytest.mark.parametrize("kw", [dict(), dict(lazy_touch=0), dict(use_graph=0, precision=1)])
-def test_narrow_edge_tiles(mplu, oracle, n, nb, edge, kw):
+def test_narrow_edge_tiles(mplu, oracle, record_property, n, nb, edge, kw):
     """opts.edge_nb: first and last block column of the left-looking schedule narrower than nb.  Other tile boundaries mean
     other rank-k pieces of the same sums: factors agree with the uniform tiling to a few 16-bit ulps, the refined solution
     is the same to fp64 accuracy, repeated runs are bit-identical."""
@@ -481,6 +499,8 @@ def test_narrow_edge_tiles(mplu, oracle, n, nb, edge, kw):
         assert (LU1 - LU0).abs().max().item() <= tol * LU0.abs().max().item()
         assert float((x1 - 1).abs().max()) < 1e-11 and float((x1 - x0).abs().max()) < 1e-11
         assert st1.backward_error <= 2 * n * EPS
+        check_factors(oracle, record_property, A, LU0, kw.get("precision", 0), "rho_reference")
+        check_factors(oracle, record_property, A, LU1, kw.get("precision", 0))
     finally:
         s.close()
 
@@ -489,7 +509,7 @@ def test_narrow_edge_tiles(mplu, oracle, n, nb, edge, kw):
                                               (3000, 1024, 1024, 6), (4096, 2048, 512, 8)])
 @pytest.mark.parametrize("precision", [0, 1])
 @pytest.mark.timeout(300)
-def test_dataflow_getrf_matches_the_launch_per_product_path(mplu, oracle, n, nb, flow_w, ctas, precision):
+def test_dataflow_getrf_matches_the_launch_per_product_path(mplu, oracle, record_property, n, nb, flow_w, ctas, precision):
     """opts.flow_w: the GETRF of a diagonal block as ONE dataflow launch (csrc/getrf_flow.cu): right-looking at 128-block
     granularity, leaf CTAs + helper CTAs that pull tile products from a priority-ordered list and hand results over through
     counters.  Same tcgen05 products on the same 16-bit operands as the recursion, but the Schur updates are summed in
@@ -518,6 +538,8 @@ def test_dataflow_getrf_matches_the_launch_per_product_path(mplu, oracle, n, nb,
         tol = 2.0 ** -8 if precision == 0 else 2.0 ** -5
         assert dU <= tol * LU0.abs().max().item(), dU
         assert dL <= tol * torch.tril(LU0, -1).abs().max().item(), dL
+        check_factors(oracle, record_property, A, LU0, precision, "rho_unfused")
+        check_factors(oracle, record_property, A, LU1, precision, "rho_dataflow")
         assert float((x1 - 1).abs().max()) < 1e-11 and float((x1 - x0).abs().max()) < 1e-11
     finally:
         s.close()
@@ -525,7 +547,7 @@ def test_dataflow_getrf_matches_the_launch_per_product_path(mplu, oracle, n, nb,
 
 @pytest.mark.parametrize("n,nb", [(4096, 1024), (2048, 512)])
 @pytest.mark.parametrize("precision", [0, 1])
-def test_lazy_first_touch_is_bit_identical(mplu, n, nb, precision):
+def test_lazy_first_touch_is_bit_identical(mplu, oracle, record_property, n, nb, precision):
     """opts.lazy_touch: no separate fp64 -> fp32 cast pass over A -- every tile's first Schur update takes its addend
     straight from the caller's fp64 matrix (the cast of /root/reference/MPF.cu:20-25,106-121 fused into the GEMM
     epilogue's loads) and ||A||_inf rides in the first residual.  Same arithmetic: identical factors, norms, solutions."""
@@ -535,6 +557,7 @@ def test_lazy_first_touch_is_bit_identical(mplu, n, nb, precision):
     try:
         x0, st0 = s.gesv(A, b, mplu.default_options(nb=nb, lazy_touch=0, precision=precision))
         LU0 = s.factors(n).clone()
+        check_factors(oracle, record_property, A, LU0, precision)
         for rep in range(2):
             x1, st1 = s.gesv(A, b, mplu.default_options(nb=nb, lazy_touch=1, precision=precision))
             assert torch.equal(s.factors(n), LU0)
@@ -549,7 +572,7 @@ def test_lazy_first_touch_is_bit_identical(mplu, n, nb, precision):
         s.close()
 
 
-def test_lazy_first_touch_scale_overflow_is_redone(mplu, oracle, solver):
+def test_lazy_first_touch_scale_overflow_is_redone(mplu, oracle, solver, record_property):
     """the fp16 scale of the lazy first touch comes from the first block column / row only; an interior block 2^6 larger
     leaves the fp16 range under it: detected, redone with the global scale, right answer"""
     import torch
@@ -558,7 +581,11 @@ def test_lazy_first_touch_scale_overflow_is_redone(mplu, oracle, solver):
     A[nb:, nb:] *= 64.0
     b = A.sum(axis=1)
     x, st = run(mplu, solver, A, b, nb=nb, lazy_touch=1)
+    if st["status_bits"] == 0:  # an overflow that did not spoil the solve keeps its factors on purpose
+        check_factors(oracle, record_property, A, solver.factors(n), 0, "rho_lazy")
     x0, st0 = run(mplu, solver, A, b, nb=nb, lazy_touch=0)
+    if st0["status_bits"] == 0:
+        check_factors(oracle, record_property, A, solver.factors(n), 0, "rho_eager")
     assert st["converged"] == 1 and st0["converged"] == 1
     np.testing.assert_allclose(x, x0, rtol=0, atol=1e-10)
     np.testing.assert_allclose(x, 1.0, rtol=0, atol=1e-9)

@@ -132,3 +132,115 @@ def test_blocked_generator_equals_counter_matrix(oracle, n, dominant):
     A = np.empty((n, n), order="F")
     oracle.counter_matrix_into(A, seed=3, dominant=dominant, block=256)
     assert np.array_equal(A, oracle.counter_matrix(n, seed=3, dominant=dominant))
+
+
+def _randn_dominant(n, seed):
+    """stable without pivoting, and its off-diagonal blocks carry O(1) weight next to a diagonal of 2 sqrt(n)"""
+    return np.random.default_rng(seed).standard_normal((n, n)) + 2.0 * np.sqrt(n) * np.eye(n)
+
+
+@pytest.mark.parametrize("n", [1024, 3000])
+@pytest.mark.parametrize("kind", ["counter", "randn"])
+def test_factor_tile_ratio_of_the_emulated_factors(oracle, n, kind):
+    """the tile-wise componentwise backward error of the emulated 16-bit factorization is a few unit roundoffs of the
+    16-bit type (the bound the GPU factor tests use is 3 u), on dominant and on randn + 2 sqrt(n) I inputs"""
+    A = oracle.counter_matrix(n, seed=1) if kind == "counter" else _randn_dominant(n, 1)
+    for bf16, u in ((False, 2.0 ** -11), (True, 2.0 ** -8)):
+        rho = oracle.factor_tile_ratio(A, oracle.lu_mixed_emulated(A, 128, bf16=bf16))
+        assert rho.shape == ((n + 127) // 128,) * 2
+        assert 0 < rho.max() <= 2 * u, (bf16, rho.max() / u)
+
+
+def test_factor_tile_ratio_names_a_wrong_tile(oracle):
+    """one off-diagonal tile of the factors 1 % off: that tile and only that tile leaves the bound, although the
+    refinement still converges and the error is far below the old normwise tolerances (2^-9 max|LU|)"""
+    n, u = 1024, 2.0 ** -11
+    A = _randn_dominant(n, 2)
+    F = oracle.lu_mixed_emulated(A, 128)
+    assert oracle.factor_tile_ratio(A, F).max() <= 3 * u
+    for I, J in ((1, 4), (5, 1)):  # a tile of U, a tile of L
+        G = F.copy()
+        G[128 * I:128 * (I + 1), 128 * J:128 * (J + 1)] *= 1.01
+        rho = oracle.factor_tile_ratio(A, G)
+        bad = np.argwhere(rho > 3 * u)
+        assert [tuple(t) for t in bad] == [(I, J)], bad
+        assert oracle.refine(A, A.sum(axis=1), G)["converged"]
+
+
+def test_factor_tile_ratio_edges(oracle):
+    # ragged order, exact factors: zero error; a tile whose |L||U| is zero must have zero error too
+    A = _randn_dominant(200, 3)
+    rho = oracle.factor_tile_ratio(A, oracle.lu_nopivot_fp64(A))
+    assert rho.shape == (2, 2) and rho.max() <= 1e-14
+    D = np.diag(np.arange(1.0, 257.0))
+    assert (oracle.factor_tile_ratio(D, D) == 0).all()  # off-diagonal tiles: M = 0 and E = 0
+    D2 = D.copy()
+    D2[200, 10] = 1.0  # A has an entry where L U (= D) has none
+    rho = oracle.factor_tile_ratio(D2, D)
+    assert rho[1, 0] == np.inf and rho[0, 0] == 0 and rho[1, 1] == 0
+    try:
+        import torch
+    except ImportError:
+        return
+    F = oracle.lu_mixed_emulated(A, 128)
+    np.testing.assert_allclose(oracle.factor_tile_ratio(torch.tensor(A), torch.tensor(F.astype(np.float64))),
+                               oracle.factor_tile_ratio(A, F), rtol=1e-12)
+
+
+def _exact_block_inverses(LU, blk=128):
+    n = LU.shape[0]
+    npad = -(-n // blk) * blk
+    F = np.eye(npad)
+    F[:n, :n] = LU
+    Li, Ui = [], []
+    for i in range(npad // blk):
+        D = F[i * blk:(i + 1) * blk, i * blk:(i + 1) * blk]
+        Li.append(np.linalg.inv(np.tril(D, -1) + np.eye(blk)))
+        Ui.append(np.linalg.inv(np.triu(D)))
+    return np.array(Li), np.array(Ui)
+
+
+@pytest.mark.parametrize("n", [1, 127, 129, 1000])
+def test_blocked_sweeps_are_the_triangular_solves(oracle, n):
+    """with exact block inverses and the solved blocks kept in fp64, the blocked sweeps are L U x = b; with fp32 blocks,
+    fp32 factors and an fp32 evaluation they stay within fp32 rounding of it"""
+    from scipy.linalg import solve_triangular
+    A = _randn_dominant(n, n)
+    LU = oracle.lu_nopivot_fp64(A)
+    Li, Ui = _exact_block_inverses(LU)
+    rng = np.random.default_rng(0)
+    B = rng.standard_normal((n, 3)).astype(np.float32).astype(np.float64)  # the sweeps take b in fp32
+    y = solve_triangular(LU, B, lower=True, unit_diagonal=True)
+    X = solve_triangular(LU, y, lower=False)
+    got = oracle.blocked_sweeps(LU, Li, Ui, B, store=np.float64)
+    np.testing.assert_allclose(got, X, rtol=0, atol=1e-12 * np.abs(X).max())
+    x1 = oracle.blocked_sweeps(LU, Li, Ui, B[:, 1], store=np.float64)
+    assert x1.shape == (n,)
+    np.testing.assert_allclose(x1, X[:, 1], rtol=0, atol=1e-12 * np.abs(X).max())
+    x64 = oracle.blocked_sweeps(LU, Li, Ui, B)  # fp32 blocks
+    x32 = oracle.blocked_sweeps(LU, Li, Ui, B, dtype=np.float32)
+    assert (x64.astype(np.float32) == x64).all() and (x32.astype(np.float32) == x32).all()
+    err = np.abs(x64 - X).max()
+    assert 0 < err <= 1e-6 * np.abs(X).max()
+    assert np.abs(x32 - X).max() <= 1e-5 * np.abs(X).max()
+
+
+def test_factor_tile_distance_sees_what_the_backward_error_bound_lets_pass(oracle):
+    """an L tile 0.1 % off stays under the 3 u backward-error bound, but against the unperturbed factors it is a
+    distance of about one u, located in its own tile; identical factors are at distance 0"""
+    n, u = 1024, 2.0 ** -11
+    A = _randn_dominant(n, 2)
+    F = oracle.lu_mixed_emulated(A, 128)
+    assert (oracle.factor_tile_distance(F, F) == 0).all()
+    G = F.copy()
+    G[640:768, 128:256] *= 1.001
+    assert oracle.factor_tile_ratio(A, G).max() <= 3 * u
+    d = oracle.factor_tile_distance(G, F)
+    assert np.unravel_index(np.argmax(d), d.shape) == (5, 1) and d.max() >= u / 2
+    assert d[:5].max() == 0 and d[6:].max() == 0  # only tile row 5 of L U changes
+    try:
+        import torch
+    except ImportError:
+        return
+    np.testing.assert_allclose(oracle.factor_tile_distance(torch.tensor(G.astype(np.float64)), torch.tensor(F.astype(np.float64))),
+                               d, rtol=1e-12)

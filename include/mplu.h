@@ -66,7 +66,8 @@ typedef struct mplu_options {
                          stream (default 0: measured much slower, 62.6 ms -- the carve-out starves the trailing GEMM) */
     int stream_host;  /* mplu_gesv_host only.  1 (default): A is copied block column by block column and factored
                          left-looking as it arrives, so the factorization hides behind the PCIe transfer (same factors
-                         bit for bit); 0: copy everything, then run the device schedule */
+                         bit for bit); 0: copy everything, then run the device schedule.  Not with equilibrate = 1: the
+                         row scales need every column of A before the first cast, so A is copied first */
     int schedule;     /* device-resident input: MPLU_SCHED_LEFT (default) = left-looking block columns with look-ahead and
                          eager updates, MPLU_SCHED_RIGHT = right-looking trailing updates with depth-1 look-ahead
                          (same factors bit for bit; n=32768: 35.8 vs 38.3 ms) */
@@ -117,6 +118,17 @@ typedef struct mplu_options {
                          default 0 because the twice as long fp32 accumulation in the tensor core costs GMRES-IR up to 5x more
                          Krylov steps on the kappa >= 1e7 systems of the condition-number sweep (DESIGN.md section 4) */
     int flow_merge_ctas; /* helpers that take inverse-merge tasks before main-list tasks; -1 (default) = a quarter of them */
+    int equilibrate;  /* factor / gesv entry points (not the block-cyclic solver, which returns MPLU_E_ARG for anything but 0).
+                         0 (default): off.  1: like LAPACK dgesvx with FACT = 'E': the power-of-two row and column scales r, c
+                         of dgeequb are computed on the device and applied by dlaqge's rule (rows if ROWCND < 0.1 or AMAX
+                         outside [SMALL, LARGE], columns if COLCND < 0.1; nothing after a zero row / column or a non-finite
+                         entry).  With scales applied, diag(r) A diag(c) is factored (exactly: powers of two) and the
+                         refinement runs against the ORIGINAL A with x = C (LU)^-1 R b corrections, so backward errors, the
+                         stopping rule and the fp64 fallback keep their meaning.  Keeps matrices with widely different row or
+                         column magnitudes inside the fp16 range.  Costs two HBM passes over A; when scales are applied the
+                         cast of A is an eager pass (lazy_touch does not apply) and mplu_gesv_host copies A before
+                         factoring (stream_host does not apply).  When no scale is applied, everything after the two passes
+                         is the equilibrate = 0 computation, bit for bit.  See mplu_get_equilibration. */
 } mplu_options;
 
 typedef struct mplu_stats {
@@ -146,6 +158,8 @@ typedef struct mplu_stats {
     int dsgesv_iter;        /* LAPACK dsgesv's ITER: >= 0 refinement iterations of a successful mixed-precision solve; < 0 the
                                fallback ran: -2 low-precision overflow, -3 low-precision factorization unusable (zero pivot),
                                -(max_iters + 1) refinement did not converge */
+    int equed;              /* opts.equilibrate: LAPACK's EQUED of the mixed-precision factorization, 0 N (no scaling), 1 R (rows),
+                               2 C (columns), 3 B (both); reported also when the fp64 fallback then solved the original system */
 } mplu_stats;
 
 void mplu_default_options(mplu_options *opts);
@@ -196,8 +210,15 @@ int mplu_gesv_host_nrhs(mplu_context *ctx, int n, int nrhs, const double *hA, lo
                         mplu_stats *stats);
 
 /* Copy the fp32 L\U factors (unit-lower L below the diagonal, U on/above: the dgetrf layout MPF returns) widened
- * to fp64 into a column-major n x n array; `on_device` selects the destination memory space. */
+ * to fp64 into a column-major n x n array; `on_device` selects the destination memory space.  After an equilibrated
+ * factorization these are the factors of diag(r) A diag(c) (mplu_get_equilibration). */
 int mplu_get_factors(mplu_context *ctx, double *LU, long long ldlu, int on_device);
+
+/* The equilibration of the last factorization (opts.equilibrate): *equed (may be null) = 0 N / 1 R / 2 C / 3 B, and the
+ * row / column scales r, c (n doubles each, may be null; `on_device` selects their memory space).  A side that was not
+ * applied reads as ones, so the factors are always those of diag(r) A diag(c).  MPLU_E_NOTFACTORED before any
+ * factorization. */
+int mplu_get_equilibration(mplu_context *ctx, int *equed, double *r, double *c, int on_device);
 
 /* The stream all work of this context is enqueued on (a cudaStream_t). */
 void *mplu_stream(mplu_context *ctx);

@@ -29,7 +29,7 @@ class Options(C.Structure):
     _fields_ = [("precision", C.c_int), ("nb", C.c_int), ("max_iters", C.c_int), ("tol", C.c_double),
                 ("gemm_variant", C.c_int), ("max_sms", C.c_int), ("a_exp", C.c_int), ("l_exp", C.c_int),
                 ("lookahead", C.c_int), ("side_sms", C.c_int), ("use_graph", C.c_int), ("pdl", C.c_int), ("group", C.c_int),
-                ("refinement", C.c_int), ("gmres_restart", C.c_int), ("gmres_tol", C.c_double), ("bf16_fallback", C.c_int), ("tile_ws", C.c_int), ("cg2_min_elems", C.c_int), ("side_sms_early", C.c_int), ("early_pct", C.c_int), ("tri_skip", C.c_int), ("late_pct", C.c_int), ("l2_persist", C.c_int), ("stream_host", C.c_int), ("schedule", C.c_int), ("eager", C.c_int), ("side_sms_left", C.c_int), ("stream_c", C.c_int), ("early_scale", C.c_int), ("fuse_w", C.c_int), ("fuse_ctas", C.c_int), ("lazy_touch", C.c_int), ("flow_w", C.c_int), ("flow_ctas", C.c_int), ("fp64_fallback", C.c_int), ("edge_nb", C.c_int), ("pair_ts", C.c_int), ("update_pair", C.c_int), ("flow_merge_ctas", C.c_int)]
+                ("refinement", C.c_int), ("gmres_restart", C.c_int), ("gmres_tol", C.c_double), ("bf16_fallback", C.c_int), ("tile_ws", C.c_int), ("cg2_min_elems", C.c_int), ("side_sms_early", C.c_int), ("early_pct", C.c_int), ("tri_skip", C.c_int), ("late_pct", C.c_int), ("l2_persist", C.c_int), ("stream_host", C.c_int), ("schedule", C.c_int), ("eager", C.c_int), ("side_sms_left", C.c_int), ("stream_c", C.c_int), ("early_scale", C.c_int), ("fuse_w", C.c_int), ("fuse_ctas", C.c_int), ("lazy_touch", C.c_int), ("flow_w", C.c_int), ("flow_ctas", C.c_int), ("fp64_fallback", C.c_int), ("edge_nb", C.c_int), ("pair_ts", C.c_int), ("update_pair", C.c_int), ("flow_merge_ctas", C.c_int), ("equilibrate", C.c_int)]
 
 
 class Stats(C.Structure):
@@ -39,7 +39,7 @@ class Stats(C.Structure):
                 ("factor_ms", C.c_float), ("solve_ms", C.c_float), ("total_ms", C.c_float),
                 ("h2d_ms", C.c_float), ("d2h_ms", C.c_float), ("gemm_launches", C.c_int),
                 ("kernel_launches", C.c_int), ("trailing_launches", C.c_int), ("trailing_ms", C.c_float),
-                ("trailing_flops", C.c_double), ("trailing_bytes", C.c_double), ("gmres_iters", C.c_int), ("precision_used", C.c_int), ("fp64_fallback", C.c_int), ("dsgesv_iter", C.c_int)]
+                ("trailing_flops", C.c_double), ("trailing_bytes", C.c_double), ("gmres_iters", C.c_int), ("precision_used", C.c_int), ("fp64_fallback", C.c_int), ("dsgesv_iter", C.c_int), ("equed", C.c_int)]
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
@@ -77,6 +77,7 @@ def load_library(path: os.PathLike | None = None) -> C.CDLL:
     lib.mplu_gesv_device.argtypes = [vp, i, vp, ll, vp, vp, C.POINTER(Options), C.POINTER(Stats)]
     lib.mplu_gesv_host.argtypes = [vp, i, vp, ll, vp, vp, C.POINTER(Options), C.POINTER(Stats)]
     lib.mplu_get_factors.argtypes = [vp, vp, ll, i]
+    lib.mplu_get_equilibration.argtypes = [vp, C.POINTER(i), vp, vp, i]
     dp = C.POINTER(C.c_double)
     lib.mplu_solve_device_nrhs.argtypes = [vp, i, vp, ll, vp, ll, vp, ll, dp, C.POINTER(Stats)]
     lib.mplu_gesv_device_nrhs.argtypes = [vp, i, i, vp, ll, vp, ll, vp, ll, C.POINTER(Options), dp, C.POINTER(Stats)]
@@ -88,7 +89,7 @@ def load_library(path: os.PathLike | None = None) -> C.CDLL:
     lib.mplu_generate.restype = i
     for name in ("mplu_create", "mplu_factor_device", "mplu_solve_device", "mplu_gesv_device", "mplu_gesv_host",
                  "mplu_get_factors", "mplu_gemm16", "mplu_diag_lu128", "mplu_residual", "mplu_solve_device_nrhs",
-                 "mplu_gesv_device_nrhs", "mplu_gesv_host_nrhs"):
+                 "mplu_gesv_device_nrhs", "mplu_gesv_host_nrhs", "mplu_get_equilibration"):
         getattr(lib, name).restype = i
     lib.mplu_MPF.argtypes = [vp, i, i, vp]
     lib.mplu_MPF.restype = i
@@ -241,6 +242,19 @@ class Solver:
         LU = torch.empty(n, n, dtype=torch.float64, device="cuda").t()  # column-major storage
         _check(self._lib.mplu_get_factors(self._ctx, LU.data_ptr(), n, 1), "mplu_get_factors")
         return LU
+
+    def equilibration(self, n):
+        """(equed, r, c) of the last factorization (opts.equilibrate): EQUED 0 N / 1 R / 2 C / 3 B and the row / column
+        scales as fp64 CUDA tensors of length n (ones on a side that was not applied); the stored factors are those of
+        diag(r) A diag(c)."""
+        import torch
+        r = torch.empty(n, dtype=torch.float64, device="cuda")
+        c = torch.empty(n, dtype=torch.float64, device="cuda")
+        equed = C.c_int()
+        torch.cuda.synchronize()
+        _check(self._lib.mplu_get_equilibration(self._ctx, C.byref(equed), r.data_ptr(), c.data_ptr(), 1),
+               "mplu_get_equilibration")
+        return equed.value, r, c
 
 
 # ---- 2D block-cyclic layout (host-side helpers; the same index maps as csrc/dist.cu) ------------------------------

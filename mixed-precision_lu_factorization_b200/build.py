@@ -27,7 +27,7 @@ NVCC_FLAGS = [
 # of the build stamp, so a plain build() afterwards rebuilds the default library
 NVCC_FLAGS += os.environ.get("MPLU_EXTRA_NVCC_FLAGS", "").split()
 
-SOURCES = ["gemm_tc.cu", "getrf_fused.cu", "getrf_flow.cu", "panel.cu", "ir.cu", "lu.cu", "gmres.cu", "dist.cu", "generate.cu", "mpf_compat.cu", "fp64_fallback.cu", "dropin_kernels.cu"]
+SOURCES = ["gemm_tc.cu", "getrf_fused.cu", "getrf_flow.cu", "panel.cu", "equil.cu", "ir.cu", "lu.cu", "gmres.cu", "dist.cu", "generate.cu", "mpf_compat.cu", "fp64_fallback.cu", "dropin_kernels.cu"]
 
 
 def _nvcc() -> str:

@@ -1209,6 +1209,7 @@ int mplu_dist_local_shape(const mplu_dist* d, int i, int n, int nb, int* p, int*
 int mplu_dist_gesv(mplu_dist* d, int n, int nb, const double* const* dA, const long long* lda,
                    const double* const* db, double* const* dx, const mplu_options* opts, mplu_stats* stats) {
     if (!d || n <= 0 || nb < kDiagBlock || nb % kDiagBlock || n % nb || !dA || !lda || !db || !dx) return MPLU_E_ARG;
+    if (opts && opts->equilibrate != 0) return MPLU_E_ARG;  // no equilibration in the block-cyclic solver
     CK(cudaSetDevice(d->device));
     if (opts) d->opts = *opts;
     d->opts.nb = nb;
@@ -1305,6 +1306,7 @@ int mplu_dist_gesv(mplu_dist* d, int n, int nb, const double* const* dA, const l
 int mplu_dist_gesv_host(mplu_dist* d, int n, int nb, const double* const* hA, const long long* lda,
                         const double* const* hb, double* const* hx, const mplu_options* opts, mplu_stats* stats) {
     if (!d || n <= 0 || nb < kDiagBlock || nb % kDiagBlock || n % nb || !hA || !lda || !hb || !hx) return MPLU_E_ARG;
+    if (opts && opts->equilibrate != 0) return MPLU_E_ARG;
     CK(cudaSetDevice(d->device));
     const size_t L = d->ranks.size();
     if (d->stA.size() != L) { d->stA.assign(L, nullptr); d->stb.assign(L, nullptr); d->stx.assign(L, nullptr); d->stA_cap.assign(L, 0); d->st_n = 0; }

@@ -1,6 +1,6 @@
 // GMRES-based iterative refinement (SURVEY.md section 8f item 3; Carson & Higham's GMRES-IR): the correction equation
 // A d = r of each refinement step is solved by GMRES in fp64, left-preconditioned with the low-precision factors,
-//     (LU)^-1 A d = (LU)^-1 r,
+//     M^-1 A d = M^-1 r,   M^-1 = (LU)^-1, or C (LU)^-1 R with equilibrated factors of diag(r) A diag(c),
 // instead of the single solve d = (LU)^-1 r of classic refinement.  The preconditioned operator is applied with the
 // kernels the classic path already has (fp64 A*v: residual kernels; (LU)^-1: lu_solve_kernel on the fp32 factors), so
 // this file only adds the Krylov bookkeeping: classical Gram-Schmidt with re-orthogonalisation on the device (two
@@ -51,10 +51,28 @@ __global__ void scale_to_kernel(const double* __restrict__ w, double a, double* 
 
 namespace mplu_detail {
 
+// out = M^-1 in for the preconditioner M^-1 = C (LU)^-1 R of the stored factors (R, C: the equilibration's scales where
+// applied, identity otherwise; eq_D is the scratch of the scaled right-hand side)
+int apply_preconditioner(mplu_context* c, const double* in, double* out) {
+    const int n = c->n;
+    cudaStream_t st = c->stream;
+    const double* rhs = in;
+    if (c->equed & 1) {
+        CKI(launch_diag_scale(c->eq_r, n, 1, in, n, c->eq_D, n, 0, st));
+        rhs = c->eq_D;
+        c->kernel_launches += 1;
+    }
+    CKI(launch_lu_solve(c->W, c->npad, n, c->npad, c->Linv32, c->Uinv32, rhs, c->y, out, nullptr, c->ready, st));
+    if (c->equed & 2) {
+        CKI(launch_diag_scale(c->eq_c, n, 1, out, n, out, n, 0, st));
+        c->kernel_launches += 1;
+    }
+    return 0;
+}
+
 // One GMRES solve of A d = r (r: n doubles on the device), x += d.  Returns 0 or an error code; *inner = Krylov steps taken.
 int gmres_correction(mplu_context* c, const double* dA, long long lda, const double* r, double* dx, int* inner) {
-    const int n = c->n, npad = c->npad;
-    const long long ld = npad;
+    const int n = c->n;
     cudaStream_t st = c->stream;
     const int m = c->opts.gmres_restart > 0 ? c->opts.gmres_restart : 50;
     const double tol = c->opts.gmres_tol > 0 ? c->opts.gmres_tol : 1e-6;
@@ -86,8 +104,8 @@ int gmres_correction(mplu_context* c, const double* dA, long long lda, const dou
         return (int)cudaStreamSynchronize(st);
     };
 
-    // z0 = (LU)^-1 r -> V[:,0]
-    CKI(launch_lu_solve(c->W, ld, n, npad, c->Linv32, c->Uinv32, r, c->y, w, nullptr, c->ready, st));
+    // z0 = M^-1 r -> V[:,0]
+    CKI(apply_preconditioner(c, r, w));
     CKI(dots(w, 0, hh.data()));
     const double beta = std::sqrt(hh[0]);
     *inner = 0;
@@ -96,9 +114,9 @@ int gmres_correction(mplu_context* c, const double* dA, long long lda, const dou
     g[0] = beta;
     int k = 0;
     for (int j = 0; j < m; ++j) {
-        // w = (LU)^-1 (A v_j):  tmp = 0 - A v_j, w = -(LU)^-1 tmp
+        // w = M^-1 (A v_j):  tmp = 0 - A v_j, w = -M^-1 tmp
         CKI(launch_residual(dA, lda, n, V + (size_t)j * n, c->gm_zero, tmp, c->partial, c->nchunk, c->norms, st));
-        CKI(launch_lu_solve(c->W, ld, n, npad, c->Linv32, c->Uinv32, tmp, c->y, w, nullptr, c->ready, st));
+        CKI(apply_preconditioner(c, tmp, w));
         scale_to_kernel<<<nb256, 256, 0, st>>>(w, -1.0, w, n);
         c->kernel_launches += 4;
         // classical Gram-Schmidt, twice

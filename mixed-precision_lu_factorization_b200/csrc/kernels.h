@@ -20,8 +20,10 @@ constexpr int kDiagBlock = 128;  // diagonal block / base panel width
 
 // panel.cu
 int panel_init();  // per-device kernel attributes; call before the first launch / graph capture
+// rscale / cscale non-null (equilibration): W = fp32(diag(rscale) A diag(cscale)), amax of that; ||A||_inf of A itself
 int launch_first_touch(const double* A, long long lda, int n, float* W, long long ldw, int npad, float* amax,
-                       double* rowsum_part, int nchunk, double* anorm, cudaStream_t st);
+                       double* rowsum_part, int nchunk, double* anorm, cudaStream_t st, const double* rscale = nullptr,
+                       const double* cscale = nullptr);
 // the same first touch for the columns [cb, ce) only (amax accumulates, not reset; row sums into slots
 // [slot0, slot0 + nslots) of rowsum_part), and the final ||A||_inf over the first nslots slots
 int launch_first_touch_cols(const double* A, long long lda, int n, float* W, long long ldw, int npad, int cb, int ce,
@@ -42,6 +44,16 @@ int launch_diag_lu(float* W, long long ldw, int k0, void* Linv16, void* Uinv16, 
                    long long* dbg_clk = nullptr,  // optional device array of phase time stamps (clock64)
                    int pdl = 0,                   // 1 = programmatic dependent launch
                    int valid = kDiagBlock);       // rows/columns of the block that belong to the matrix (the rest is identity padding)
+
+// equil.cu: dgeequb scales + dlaqge decision.  eq: EQ_WORDS device words; the non-negative doubles are kept as bit patterns.
+enum EquilWord : int { EQ_RMIN = 0, EQ_CMIN = 1, EQ_RMAX = 2, EQ_CMAX = 3, EQ_BAD = 4, EQ_EQUED = 5, EQ_WORDS = 8 };
+// r (n), c (n) = the scales of the applied sides, 1 elsewhere; eq[EQ_EQUED] = EQUED (bit 0 rows, bit 1 columns; 0 after a
+// zero row / column or a non-finite entry).  part: nchunk * n doubles of workspace.  Four launches.
+int launch_equilibrate(const double* A, long long lda, int n, double* part, int nchunk, double* r, double* c,
+                       unsigned long long* eq, cudaStream_t st);
+// out(:, j) = s o in(:, j) (accumulate: out(:, j) += s o in(:, j)) for k columns; in may be out
+int launch_diag_scale(const double* s, int n, int k, const double* in, long long ldi, double* out, long long ldo,
+                      int accumulate, cudaStream_t st);
 
 // ir.cu
 // r = b - A*x (fp64), ||r||_inf and ||x||_inf into norms[0], norms[1]

@@ -71,6 +71,37 @@ int ensure_rhs_work(mplu_context* c, int nrhs) {
     return 0;
 }
 
+int ensure_equil_scratch(mplu_context* c, size_t elems) {
+    if (elems <= c->eq_D_cap) return 0;
+    cudaFree(c->eq_D);
+    c->eq_D = nullptr; c->eq_D_cap = 0;
+    CK(cudaMalloc(&c->eq_D, elems * sizeof(double)));
+    c->eq_D_cap = elems;
+    return 0;
+}
+
+// opts.equilibrate = 1: dgeequb's scales of A into c->eq_r / c->eq_c and dlaqge's EQUED into c->equed.  The host needs
+// EQUED to choose the first touch, so it is read back here (one synchronisation, before any graph launch).
+int equilibrate(mplu_context* c, const double* dA, long long lda) {
+    const int n = c->n;
+    cudaStream_t st = c->stream;
+    if (n > c->eq_cap_n) {
+        cudaFree(c->eq_r); cudaFree(c->eq_c);
+        c->eq_r = c->eq_c = nullptr; c->eq_cap_n = 0;
+        CK(cudaMalloc(&c->eq_r, (size_t)n * sizeof(double)));
+        CK(cudaMalloc(&c->eq_c, (size_t)n * sizeof(double)));
+        c->eq_cap_n = n;
+    }
+    if (!c->eq_words) CK(cudaMalloc(&c->eq_words, EQ_WORDS * sizeof(unsigned long long)));
+    // rowsum_part (nchunk x npad) is free until the first touch: the row pass keeps its per-chunk maxima there
+    CKI(launch_equilibrate(dA, lda, n, c->rowsum_part, c->nchunk, c->eq_r, c->eq_c, c->eq_words, st));
+    unsigned long long equed = 0;
+    CK(cudaMemcpyAsync(&equed, c->eq_words + EQ_EQUED, sizeof(equed), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    c->equed = (int)equed;
+    return 0;
+}
+
 int effective_nb(const mplu_context* c, int npad) {
     int NB = c->opts.nb;
     if (NB < kDiagBlock) NB = kDiagBlock;
@@ -1460,6 +1491,15 @@ int factor_impl(mplu_context* c, int n, const double* dA, long long lda) {
     const int npad = c->npad;
     cudaStream_t st = c->stream;
     CK(cudaMemsetAsync(c->status, 0, sizeof(int), st));
+    // Equilibration: with scales to apply, W = diag(r) A diag(c) comes from the eager first touch (the lazy one and the
+    // early-scale prologue read A itself); the captured schedule is the same.  EQUED = N changes nothing below.
+    c->equed = 0;
+    int eq_kern = 0;
+    if (c->opts.equilibrate == 1) {
+        CKI(equilibrate(c, dA, lda));
+        eq_kern = 4;
+    }
+    const bool scaled = c->equed != 0;
     // left-looking schedule with at least two block columns: the first touch overlaps the first diagonal tile
     // Lazy first touch (left-looking schedule, order a multiple of 128, at least two block columns): only the first
     // block column and block row are cast here; every other tile's first update reads its addend from the fp64 matrix
@@ -1467,10 +1507,10 @@ int factor_impl(mplu_context* c, int n, const double* dA, long long lda) {
     // panels; a later entry that leaves the fp16 range under it raises the overflow bit and the caller redoes the
     // factorization with the full first touch and the global scale (allow_early = false), like early_scale.
     const int NB0 = effective_nb(c, npad);
-    const bool lazy = c->opts.schedule == MPLU_SCHED_LEFT && c->opts.lazy_touch != 0 && c->allow_early && npad == n &&
-                      npad > NB0 && c->opts.tile_ws == 0 && !c->trace;
-    const bool early = !lazy && c->opts.schedule == MPLU_SCHED_LEFT && c->opts.early_scale != 0 && c->allow_early &&
-                       npad > NB0 && c->opts.tile_ws == 0;
+    const bool lazy = !scaled && c->opts.schedule == MPLU_SCHED_LEFT && c->opts.lazy_touch != 0 && c->allow_early &&
+                      npad == n && npad > NB0 && c->opts.tile_ws == 0 && !c->trace;
+    const bool early = !scaled && !lazy && c->opts.schedule == MPLU_SCHED_LEFT && c->opts.early_scale != 0 &&
+                       c->allow_early && npad > NB0 && c->opts.tile_ws == 0;
     c->lazy = lazy;
     c->anorm_pending = lazy;
     c->prologue_done = early;
@@ -1490,7 +1530,8 @@ int factor_impl(mplu_context* c, int n, const double* dA, long long lda) {
         pro_gemm = c->gemm_launches;
         pro_kern = c->kernel_launches;
     } else {
-        CKI(launch_first_touch(dA, lda, n, c->W, npad, npad, c->amax, c->rowsum_part, c->nchunk, c->anorm, st));
+        CKI(launch_first_touch(dA, lda, n, c->W, npad, npad, c->amax, c->rowsum_part, c->nchunk, c->anorm, st,
+                               scaled ? c->eq_r : nullptr, scaled ? c->eq_c : nullptr));
     }
 
     const bool use_graph = c->opts.use_graph != 0;
@@ -1543,7 +1584,7 @@ int factor_impl(mplu_context* c, int n, const double* dA, long long lda) {
         CK(cudaGraphLaunch(c->graph_exec, st));
     }
     c->gemm_launches += pro_gemm;
-    c->kernel_launches += pro_kern;
+    c->kernel_launches += pro_kern + eq_kern;
     c->factored = true;
     return 0;
 }
@@ -1559,6 +1600,8 @@ int factor_impl(mplu_context* c, int n, const double* dA, long long lda) {
 // The fp16 scale has to be fixed before the first cast: it is taken from the first block column (which holds the
 // first diagonal tile); a later block column that leaves the fp16 range under that scale sets the overflow bit and
 // the caller redoes the solve from the (by then resident) device copy with the global scale.
+// Equilibration (opts.equilibrate) is not streamed: a row scale needs every column of its row before the first cast,
+// so with it gesv_host_impl copies A first and runs the device path.
 bool streamed_supported(const mplu_context* c, int n) {
     const int npad = ((n + kDiagBlock - 1) / kDiagBlock) * kDiagBlock;
     const int NB = effective_nb(c, npad);
@@ -1575,6 +1618,7 @@ int factor_streamed(mplu_context* c, int n, const double* hA, long long lda, dou
     const int nt = (npad + NB - 1) / NB;
     const int per = c->nchunk / nt;  // row-sum slots per block column
     if (per < 1 || nt >= mplu_context::kMaxSteps) return MPLU_E_ARG;
+    c->equed = 0;  // equilibration needs all of A before the first cast: gesv_host_impl does not stream then
     cudaStream_t st = c->stream, cp = c->copy;
     CK(cudaMemsetAsync(c->status, 0, sizeof(int), st));
     CK(cudaMemsetAsync(c->amax, 0, sizeof(float), st));
@@ -1716,8 +1760,8 @@ int solve_impl(mplu_context* c, const double* dA, long long lda, const RhsBlock&
     if (k > 1) CKI(ensure_rhs_work(c, k));
     double* R = k == 1 ? c->r : c->rb_R;  // the residual columns (ld n)
     double* norms = k == 1 ? c->norms : c->rb_norms;
-    // D = (LU)^-1 rhs: D -> d_out, or x_accum += D (both with ld b.ldx)
-    auto solve = [&](const double* rhs, long long ldr, double* d_out, double* x_accum) -> int {
+    // D = (LU)^-1 rhs: D -> d_out, or x_accum += D (both with ld ldo)
+    auto solve = [&](const double* rhs, long long ldr, double* d_out, double* x_accum, long long ldo) -> int {
         if (k == 1) {
             c->kernel_launches += 1;
             return launch_lu_solve(c->W, ld, n, npad, c->Linv32, c->Uinv32, rhs, c->y, d_out, x_accum, c->ready, st);
@@ -1725,11 +1769,19 @@ int solve_impl(mplu_context* c, const double* dA, long long lda, const RhsBlock&
         for (int j0 = 0; j0 < k; j0 += kSolveBlock) {
             const int kc = std::min(kSolveBlock, k - j0);
             CKI(launch_lu_solve_block(c->W, ld, n, npad, c->Linv32, c->Uinv32, rhs + (long long)j0 * ldr, ldr, kc, c->rb_y,
-                                      d_out ? d_out + (long long)j0 * b.ldx : nullptr, b.ldx,
-                                      x_accum ? x_accum + (long long)j0 * b.ldx : nullptr, b.ldx, c->ready, st));
+                                      d_out ? d_out + (long long)j0 * ldo : nullptr, ldo,
+                                      x_accum ? x_accum + (long long)j0 * ldo : nullptr, ldo, c->ready, st));
             c->kernel_launches += 2;
         }
         return 0;
+    };
+    // equilibrated factors (of diag(r) A diag(c)): every solve with them is C (LU)^-1 R, through the n x k scratch D
+    const bool eq_rows = c->equed & 1, eq_cols = c->equed & 2;
+    if (c->equed) CKI(ensure_equil_scratch(c, (size_t)n * k));
+    double* D = c->eq_D;
+    auto scale = [&](const double* s, const double* in, long long ldi, double* out, long long ldo, int accumulate) -> int {
+        c->kernel_launches += 1;
+        return launch_diag_scale(s, n, k, in, ldi, out, ldo, accumulate, st);
     };
     RefineOps ops;
     ops.norms = norms;
@@ -1738,7 +1790,12 @@ int solve_impl(mplu_context* c, const double* dA, long long lda, const RhsBlock&
     ops.first_solve = [&]() -> int {
         CKI(launch_column_absmax(b.B, b.ldb, n, k, norms + 2 * k, st));
         c->kernel_launches += 1;
-        return solve(b.B, b.ldb, b.X, nullptr);
+        if (!eq_rows) CKI(solve(b.B, b.ldb, b.X, nullptr, b.ldx));
+        else {
+            CKI(scale(c->eq_r, b.B, b.ldb, D, n, 0));
+            CKI(solve(D, n, b.X, nullptr, b.ldx));
+        }
+        return eq_cols ? scale(c->eq_c, b.X, b.ldx, b.X, b.ldx, 0) : 0;
     };
     ops.residual = [&](bool* formed_anorm) -> int {
         // lazy first touch: ||A||_inf rides in the first residual pass (of the first column block): it streams A anyway
@@ -1762,7 +1819,14 @@ int solve_impl(mplu_context* c, const double* dA, long long lda, const RhsBlock&
         return 0;
     };
     ops.correct = [&](int* krylov_steps) -> int {
-        if (c->opts.refinement != MPLU_REFINE_GMRES) return solve(R, n, nullptr, b.X);
+        if (c->opts.refinement != MPLU_REFINE_GMRES) {
+            // R is recomputed by the next residual pass, so it is scaled in place; without C the correction accumulates
+            // straight into X
+            if (eq_rows) CKI(scale(c->eq_r, R, n, R, n, 0));
+            if (!eq_cols) return solve(R, n, nullptr, b.X, b.ldx);
+            CKI(solve(R, n, D, nullptr, n));
+            return scale(c->eq_c, D, n, b.X, b.ldx, 1);
+        }
         for (int j = 0; j < k; ++j) {
             int inner = 0;
             CKI(gmres_correction(c, dA, lda, R + (long long)j * n, b.X + (long long)j * b.ldx, &inner));
@@ -1778,6 +1842,7 @@ int solve_impl(mplu_context* c, const double* dA, long long lda, const RhsBlock&
     refine_stats(res, n, b.berr, stats);
     if (stats) {
         stats->status_bits = h_status;
+        stats->equed = c->equed;
         stats->gmres_iters = res.gmres_iters;
         stats->gemm_launches = c->gemm_launches;
         stats->kernel_launches = c->kernel_launches;
@@ -1880,7 +1945,7 @@ int gesv_host_impl(mplu_context* c, int n, const double* hA, long long lda, cons
     CK(cudaEventRecord(c->ev[3], st));
     int rc;
     float h2d = 0.f;
-    if (c->opts.stream_host && streamed_supported(c, n)) {
+    if (c->opts.stream_host && c->opts.equilibrate == 0 && streamed_supported(c, n)) {
         // block columns are factored as they arrive (factor_streamed); the staged copy of A stays for the residuals
         if (stats) memset(stats, 0, sizeof(*stats));
         c->factored = false;
@@ -1933,6 +1998,9 @@ int gesv_host_impl(mplu_context* c, int n, const double* hA, long long lda, cons
     }
     return rc;
 }
+
+// option values the entry points check (null: the context's options, already checked)
+bool options_valid(const mplu_options* o) { return !o || o->equilibrate == 0 || o->equilibrate == 1; }
 
 // the regions spanned by the columns of B and X (first to last element) share an address: X would overwrite B
 bool columns_overlap(const double* B, long long ldb, const double* X, long long ldx, int n, int nrhs) {
@@ -1987,6 +2055,7 @@ void mplu_default_options(mplu_options* o) {
     o->edge_nb = 0;
     o->pair_ts = 0;
     o->update_pair = 0;
+    o->equilibrate = 0;
 }
 
 int mplu_create(mplu_context** out, int device) {
@@ -2033,6 +2102,7 @@ void mplu_destroy(mplu_context* c) {
     cudaFree(c->scales); cudaFree(c->amax); cudaFree(c->anorm); cudaFree(c->norms); cudaFree(c->status); cudaFree(c->ready);
     cudaFree(c->dA_stage); cudaFree(c->db_stage); cudaFree(c->dx_stage);
     cudaFree(c->gm_V); cudaFree(c->gm_w); cudaFree(c->gm_h); cudaFree(c->gm_zero); cudaFree(c->aref);
+    cudaFree(c->eq_r); cudaFree(c->eq_c); cudaFree(c->eq_words); cudaFree(c->eq_D);
     if (c->tile) { mplu_destroy(c->tile); c->tile = nullptr; }
     for (auto& e : c->ev) if (e) cudaEventDestroy(e);
     for (auto& e : c->trail_ev) if (e) cudaEventDestroy(e);
@@ -2052,7 +2122,7 @@ void mplu_destroy(mplu_context* c) {
 void* mplu_stream(mplu_context* c) { return c ? (void*)c->stream : nullptr; }
 
 int mplu_factor_device(mplu_context* c, int n, const double* dA, long long lda, const mplu_options* opts) {
-    if (!c || !dA || n <= 0 || lda < n) return MPLU_E_ARG;
+    if (!c || !dA || n <= 0 || lda < n || !options_valid(opts)) return MPLU_E_ARG;
     CK(cudaSetDevice(c->device));
     if (opts) c->opts = *opts;
     const OptionsScope scope(c);
@@ -2074,13 +2144,13 @@ int mplu_solve_device(mplu_context* c, const double* dA, long long lda, const do
 
 int mplu_gesv_device(mplu_context* c, int n, const double* dA, long long lda, const double* db, double* dx,
                      const mplu_options* opts, mplu_stats* stats) {
-    if (!c || !dA || !db || !dx || n <= 0 || lda < n) return MPLU_E_ARG;
+    if (!c || !dA || !db || !dx || n <= 0 || lda < n || !options_valid(opts)) return MPLU_E_ARG;
     return gesv_device_impl(c, n, dA, lda, RhsBlock{1, db, n, dx, n, nullptr}, opts, stats);
 }
 
 int mplu_gesv_host(mplu_context* c, int n, const double* hA, long long lda, const double* hb, double* hx,
                    const mplu_options* opts, mplu_stats* stats) {
-    if (!c || !hA || !hb || !hx || n <= 0 || lda < n) return MPLU_E_ARG;
+    if (!c || !hA || !hb || !hx || n <= 0 || lda < n || !options_valid(opts)) return MPLU_E_ARG;
     return gesv_host_impl(c, n, hA, lda, RhsBlock{1, hb, n, hx, n, nullptr}, opts, stats);
 }
 
@@ -2095,14 +2165,14 @@ int mplu_solve_device_nrhs(mplu_context* c, int nrhs, const double* dA, long lon
 
 int mplu_gesv_device_nrhs(mplu_context* c, int n, int nrhs, const double* dA, long long lda, const double* dB, long long ldb,
                           double* dX, long long ldx, const mplu_options* opts, double* berr, mplu_stats* stats) {
-    if (!c || !dA || !dB || !dX || n <= 0 || nrhs < 1 || lda < n || ldb < n || ldx < n) return MPLU_E_ARG;
+    if (!c || !dA || !dB || !dX || n <= 0 || nrhs < 1 || lda < n || ldb < n || ldx < n || !options_valid(opts)) return MPLU_E_ARG;
     if (columns_overlap(dB, ldb, dX, ldx, n, nrhs)) return MPLU_E_ARG;
     return gesv_device_impl(c, n, dA, lda, RhsBlock{nrhs, dB, ldb, dX, ldx, berr}, opts, stats);
 }
 
 int mplu_gesv_host_nrhs(mplu_context* c, int n, int nrhs, const double* hA, long long lda, const double* hB, long long ldb,
                         double* hX, long long ldx, const mplu_options* opts, double* berr, mplu_stats* stats) {
-    if (!c || !hA || !hB || !hX || n <= 0 || nrhs < 1 || lda < n || ldb < n || ldx < n) return MPLU_E_ARG;
+    if (!c || !hA || !hB || !hX || n <= 0 || nrhs < 1 || lda < n || ldb < n || ldx < n || !options_valid(opts)) return MPLU_E_ARG;
     if (columns_overlap(hB, ldb, hX, ldx, n, nrhs)) return MPLU_E_ARG;
     return gesv_host_impl(c, n, hA, lda, RhsBlock{nrhs, hB, ldb, hX, ldx, berr}, opts, stats);
 }
@@ -2126,6 +2196,23 @@ int mplu_get_factors(mplu_context* c, double* LU, long long ldlu, int on_device)
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
     if (tmp) cudaFree(tmp);
     return (int)e;
+}
+
+int mplu_get_equilibration(mplu_context* c, int* equed, double* r, double* cs, int on_device) {
+    if (!c) return MPLU_E_ARG;
+    if (!c->factored) return MPLU_E_NOTFACTORED;
+    CK(cudaSetDevice(c->device));
+    const int n = c->n;
+    if (equed) *equed = c->equed;
+    const std::vector<double> ones(c->equed ? 0 : (size_t)n, 1.0);  // no scale applied: r = c = 1
+    const cudaMemcpyKind kind = on_device ? (c->equed ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice)
+                                          : (c->equed ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost);
+    const double* src[2] = {c->equed ? c->eq_r : ones.data(), c->equed ? c->eq_c : ones.data()};
+    double* dst[2] = {r, cs};
+    for (int i = 0; i < 2; ++i)
+        if (dst[i]) CK(cudaMemcpyAsync(dst[i], src[i], (size_t)n * sizeof(double), kind, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------ kernel hooks

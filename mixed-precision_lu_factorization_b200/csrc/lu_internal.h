@@ -53,6 +53,14 @@ struct mplu_context {
     double* rb_norms = nullptr;    // per column ||r||, ||x||, then ||b|| per column
     float* rb_y = nullptr;         // 2 * npad * kSolveBlock (the batched solve's fp32 work blocks)
     int rb_cap_n = 0, rb_cap_npad = 0, rb_cap_nrhs = 0;
+    // equilibration (opts.equilibrate, equil.cu): the scales of the stored factors (W holds diag(eq_r) A diag(eq_c)) and
+    // EQUED (bit 0 rows, bit 1 columns applied); eq_D = n x eq_cap_k correction scratch, allocated on first use
+    int equed = 0;
+    double* eq_r = nullptr; double* eq_c = nullptr;
+    unsigned long long* eq_words = nullptr;
+    int eq_cap_n = 0;
+    double* eq_D = nullptr;
+    size_t eq_D_cap = 0;
     // GMRES-IR workspace (gmres.cu)
     double* gm_V = nullptr; double* gm_w = nullptr; double* gm_h = nullptr; double* gm_zero = nullptr;
     int gm_cap_n = 0, gm_cap_m = 0;
@@ -190,6 +198,8 @@ int getrf_resident_tile(mplu_context* c, cudaStream_t st, int w);
 int ensure_work(mplu_context* c, int n);
 // GMRES-IR: solve A d = r (n doubles on the device) by GMRES preconditioned with the stored factors, x += d (gmres.cu)
 int gmres_correction(mplu_context* c, const double* dA, long long lda, const double* r, double* dx, int* inner);
+// eq_D holds at least `elems` doubles
+int ensure_equil_scratch(mplu_context* c, size_t elems);
 // dsgesv-style full-precision redo of a solve the low-precision factors could not deliver (fp64_fallback.cu); `why` is the
 // MPLU_E_* code the mixed-precision path ended with.  nrhs column-major right-hand sides (B, ldb) and solutions (X, ldx):
 // one fp64 factorization, then every column is solved and refined on its own; berr (host, may be null) receives each

@@ -29,9 +29,13 @@ __device__ __forceinline__ void atomic_max_float_nonneg(float* addr, float v) {
 // first touch: W = fp32(A) on [0,n)^2, identity on the padding diagonal, zero elsewhere in the padding.
 // grid: (ceil(npad/256), NCHUNK); block 256 threads; thread = one row, loops over its column chunk of [cb, ce).
 // Row sums of chunk y go to slot slot0 + y of rowsum_part (the streamed host path touches one block column at a time).
+// kScaled (equilibration, csrc/equil.cu): W = fp32(rscale_i a_ij cscale_j) and amax over those scaled values; the row sums stay
+// those of the unscaled |a_ij| (||A||_inf of the caller's matrix).  The scales are powers of two, so the product is exact.
+template <bool kScaled>
 __global__ void first_touch_kernel(const double* __restrict__ A, long long lda, int n, float* __restrict__ W,
                                    long long ldw, int npad, int cb, int ce, int slot0, float* amax,
-                                   double* rowsum_part, int rend) {
+                                   double* rowsum_part, int rend, const double* __restrict__ rscale = nullptr,
+                                   const double* __restrict__ cscale = nullptr) {
     const int row = blockIdx.x * blockDim.x + threadIdx.x;
     if (row >= rend) npad = 0;  // rows beyond rend are not touched (block-row variant); the block still reduces amax
     const int nchunk = gridDim.y;
@@ -41,12 +45,17 @@ __global__ void first_touch_kernel(const double* __restrict__ A, long long lda, 
     float lmax = 0.f;
     double rs = 0.0;
     if (row < npad) {
+        double ri = 1.0;
+        if constexpr (kScaled) ri = row < n ? __ldg(rscale + row) : 1.0;
 #pragma unroll 4
         for (int c = c0; c < c1; ++c) {
             float w;
             if (row < n && c < n) {
                 const double a = __ldg(A + row + (long long)c * lda);
-                w = static_cast<float>(a);
+                if constexpr (kScaled)
+                    w = static_cast<float>(ri * a * __ldg(cscale + c));
+                else
+                    w = static_cast<float>(a);
                 rs += fabs(a);
                 lmax = fmaxf(lmax, fabsf(w));
             } else {
@@ -157,10 +166,15 @@ diag_lu_kernel(float* __restrict__ W, long long ldw, int k0, void* __restrict__ 
 
 // ---------------------------------------------------------------------------------------------------------------
 int launch_first_touch(const double* A, long long lda, int n, float* W, long long ldw, int npad, float* amax,
-                       double* rowsum_part, int nchunk, double* anorm, cudaStream_t st) {
+                       double* rowsum_part, int nchunk, double* anorm, cudaStream_t st, const double* rscale,
+                       const double* cscale) {
     cudaMemsetAsync(amax, 0, sizeof(float), st);
     dim3 grid((npad + 255) / 256, nchunk);
-    first_touch_kernel<<<grid, 256, 0, st>>>(A, lda, n, W, ldw, npad, 0, npad, 0, amax, rowsum_part, npad);
+    if (rscale)
+        first_touch_kernel<true><<<grid, 256, 0, st>>>(A, lda, n, W, ldw, npad, 0, npad, 0, amax, rowsum_part, npad, rscale,
+                                                       cscale);
+    else
+        first_touch_kernel<false><<<grid, 256, 0, st>>>(A, lda, n, W, ldw, npad, 0, npad, 0, amax, rowsum_part, npad);
     cudaMemsetAsync(anorm, 0, sizeof(double), st);
     anorm_kernel<<<(n + 255) / 256, 256, 0, st>>>(rowsum_part, n, nchunk, anorm);
     return (int)cudaGetLastError();
@@ -170,7 +184,7 @@ int launch_first_touch_cols(const double* A, long long lda, int n, float* W, lon
                             float* amax, double* rowsum_part, int slot0, int nslots, cudaStream_t st) {
     if (ce <= cb || nslots <= 0) return 0;
     dim3 grid((npad + 255) / 256, nslots);
-    first_touch_kernel<<<grid, 256, 0, st>>>(A, lda, n, W, ldw, npad, cb, ce, slot0, amax, rowsum_part, npad);
+    first_touch_kernel<false><<<grid, 256, 0, st>>>(A, lda, n, W, ldw, npad, cb, ce, slot0, amax, rowsum_part, npad);
     return (int)cudaGetLastError();
 }
 
@@ -178,7 +192,7 @@ int launch_first_touch_block(const double* A, long long lda, int n, float* W, lo
                              float* amax, cudaStream_t st) {
     if (ce <= cb || rows <= 0) return 0;
     dim3 grid((rows + 255) / 256, 64);
-    first_touch_kernel<<<grid, 256, 0, st>>>(A, lda, n, W, ldw, npad, cb, ce, 0, amax, nullptr, rows);
+    first_touch_kernel<false><<<grid, 256, 0, st>>>(A, lda, n, W, ldw, npad, cb, ce, 0, amax, nullptr, rows);
     return (int)cudaGetLastError();
 }
 
